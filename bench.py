@@ -29,6 +29,9 @@ val.py:378-383).  Metric: images/s.
              D2H of the loss, achieved fraction of the tensor peak on the algorithmic 3x-forward FLOPs, and the CPU
              restatement of train.py --device cpu beside it
 
+--dump-outputs DIR writes what the timed step returned for its last batch (detections.npy, detections_per_image.npy): the
+inputs and weights are seeded, so two builds can be compared output for output.
+
 --impl reference runs that CPU arm alone (rank 0 only under torchrun).  N>1 = independent replicas, one
 b16 batch per GPU (the path shards by image batch, no data-path collective): weak scaling.
 """
@@ -69,6 +72,7 @@ def parse():
     ap.add_argument("--no-extra-models", action="store_true", help="skip the yolov5m b16 inference line (`extra.yolov5m_b16_inference`)")
     ap.add_argument("--no-parity-gate", action="store_true", help="skip the engine-vs-oracle check of the benchmarked plan")
     ap.add_argument("--slots", type=int, default=2, help="batches in flight per GPU, one stream + one plan each (DetectPipeline slots)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the detections of the last timed step to DIR/*.npy")
     return ap.parse_args()
 
 
@@ -620,6 +624,18 @@ def eager_torch_arm(model_cpu, x_u8_dev, steps, warmup):
 # ------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------
+def dump_outputs(out_dir, packed, counts, batch):
+    """What a caller of the timed step receives for one batch: detections.npy = the rows (cx, cy, l, s, theta, conf, cls) of
+    every image, image after image; detections_per_image.npy = how many rows belong to each image."""
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    n = counts[:batch].cpu().numpy()
+    rows = packed.cpu().numpy()
+    np.save(out / "detections.npy", np.concatenate([rows[b, :k] for b, k in enumerate(n)]).astype(np.float32))
+    np.save(out / "detections_per_image.npy", n.astype(np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -741,6 +757,8 @@ def run_ours(args):
         if rows[B] > dd[2] or min(rows) < 0:
             raise RuntimeError("NMS candidate capacity exceeded in the timed steps: the measurement would be invalid")
     det_per_img = float(sum(rows[:B])) / B
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dets[0], dets[1], B)   # the last timed step's batch
     ms_step = ms_total / args.steps
     # the same step with one batch in flight (for the comparison with earlier rounds, and as the step the per-launch
     # roofline shares refer to)

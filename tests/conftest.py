@@ -2,8 +2,6 @@ import os
 import sys
 from pathlib import Path
 
-import pytest
-
 ROOT = Path(__file__).resolve().parents[1]
 if str(ROOT) not in sys.path:
     sys.path.insert(0, str(ROOT))
@@ -11,13 +9,3 @@ if str(ROOT) not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-
-
-@pytest.fixture(scope="session")
-def ref_ext():
-    """The reference's own NMS kernels compiled from /root/reference into oracle/_ref (pinning)."""
-    from oracle.build_ref import load_ref
-    try:
-        return load_ref()
-    except (FileNotFoundError, OSError, ImportError) as e:  # pragma: no cover
-        pytest.skip(f"oracle/_ref not available: {e}")

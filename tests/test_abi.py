@@ -51,8 +51,8 @@ def test_devkit_cpp_symbols_exported():
     out = subprocess.run(["nm", "-D", "--defined-only", "-C", str(so)], capture_output=True, text=True).stdout
     assert "_poly_nms(int*, int*, float const*, int, int, float, int)" in out
     assert "_overlaps(float*, float const*, float const*, int, int, int)" in out
-    ref = ROOT / "oracle" / "_ref" / "libref_polygpu_nms.so"
-    if ref.exists():  # same mangled symbol as the reference's own object file
-        mangled = lambda p: set(re.findall(r" T (_Z9_\w+)", subprocess.run(["nm", "-D", "--defined-only", str(p)],
-                                                                            capture_output=True, text=True).stdout))
-        assert mangled(ref) <= mangled(so)
+    # the same mangled symbols as the reference's own objects define (nm -D of poly_nms_kernel.cu / poly_overlaps_kernel.cu
+    # compiled by oracle/build_ref.build_polygpu)
+    mangled = set(re.findall(r" T (_Z9_\w+)", subprocess.run(["nm", "-D", "--defined-only", str(so)],
+                                                            capture_output=True, text=True).stdout))
+    assert {"_Z9_poly_nmsPiS_PKfiifi", "_Z9_overlapsPfPKfS1_iii"} <= mangled

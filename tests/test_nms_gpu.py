@@ -1,13 +1,13 @@
 """GPU parity tests for the rotated-NMS path, called through the C ABI (ctypes -> liby5obb.so).
 
 Oracles, strongest first:
-  1. oracle/_ref — the reference's own kernels compiled from /root/reference for sm_100a
-     (nms_rotated_cuda = K1 + host scan, and the single_box_iou_rotated device function): bit-exact.
+  1. the reference's own kernels compiled for sm_100a (nms_rotated_cuda = K1 + host scan, and the
+     single_box_iou_rotated device function): bit-exact.  Their outputs on the seeded inputs below are stored in
+     tests/golden/ref_kernels_golden.npz (tests/refgolden.py).
   2. oracle/liboracle.so — scalar C++ restatement (no FMA): IoU within 1e-5, keep lists equal on
      inputs whose decisive IoUs are not within 1e-4 of the threshold.
   3. tests/golden/*.npz — fixtures produced by the reference CPU extension (tests/golden/make_golden.py).
 """
-import ctypes
 from pathlib import Path
 
 import numpy as np
@@ -16,6 +16,7 @@ import torch
 
 import oracle
 from tests.boxgen import rboxes, degenerate_pairs
+from tests.refgolden import assert_bit_equal, keep_from_bits, ref
 
 pytestmark = pytest.mark.gpu
 
@@ -23,25 +24,14 @@ ROOT = Path(__file__).resolve().parents[1]
 DEV = "cuda:0"
 
 
+KEEP_CASES = [(1, 100, 0), (63, 200, 1), (64, 200, 2), (65, 200, 3), (1000, 300, 4), (5000, 1024, 5), (30000, 1024, 6),
+              (4097, 16384, 7)]
+THRESHOLDS = [0.1, 0.2, 0.45, 0.7]
+
+
 def _nms(d, s, thr, **kw):
     from yolov5_obb_b200.nms_rotated import nms_rotated
     return nms_rotated(torch.from_numpy(d).to(DEV), torch.from_numpy(s).to(DEV), thr, **kw).cpu().numpy()
-
-
-def _ref_iou_pairs(a, b):
-    so = ROOT / "oracle" / "_ref" / "libref_iou.so"
-    if not so.exists():
-        pytest.skip("oracle/_ref/libref_iou.so not built")
-    L = ctypes.CDLL(str(so))
-    L.ref_iou_pairs.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_long, ctypes.c_void_p]
-    L.ref_iou_pairs.restype = ctypes.c_int
-    ta, tb = torch.from_numpy(a).to(DEV).contiguous(), torch.from_numpy(b).to(DEV).contiguous()
-    out = torch.empty(a.shape[0], dtype=torch.float32, device=DEV)
-    torch.cuda.synchronize()
-    rc = L.ref_iou_pairs(ta.data_ptr(), tb.data_ptr(), out.data_ptr(), a.shape[0], None)
-    assert rc == 0
-    torch.cuda.synchronize()
-    return out.cpu().numpy()
 
 
 def _our_iou_pairs(a, b):
@@ -68,16 +58,15 @@ def _near_pairs(n, seed, theta_grid):
 @pytest.mark.parametrize("theta_grid", [True, False])
 def test_iou_bitexact_vs_reference_device_function(theta_grid):
     a, b = _near_pairs(400_000, 11, theta_grid)
-    ours, ref = _our_iou_pairs(a, b), _ref_iou_pairs(a, b)
-    assert (ref > 0).mean() > 0.5, "pairs should mostly overlap"
-    bad = np.flatnonzero(ours.view(np.uint32) != ref.view(np.uint32))
-    assert bad.size == 0, f"{bad.size} of {a.shape[0]} IoUs differ bitwise; first {bad[:5]}: {ours[bad[:5]]} vs {ref[bad[:5]]}"
+    ours = _our_iou_pairs(a, b)
+    assert_bit_equal(ours, f"iou/{int(theta_grid)}")
+    assert (ours > 0).mean() > 0.5, "pairs should mostly overlap"
 
 
 def test_iou_degenerate_bitexact_and_vs_cpu_oracle():
     a, b = degenerate_pairs()
-    ours, ref = _our_iou_pairs(a, b), _ref_iou_pairs(a, b)
-    assert np.array_equal(ours.view(np.uint32), ref.view(np.uint32)), (ours, ref)
+    ours, want = _our_iou_pairs(a, b), ref("iou_degenerate")
+    assert np.array_equal(ours.view(np.uint32), want.view(np.uint32)), (ours, want)
     # the CPU restatement agrees except on the last 4 pairs (one rectangle written two ways: all edges
     # parallel/coincident), where FMA contraction changes which candidate points survive — there the
     # reference's own CPU and CUDA builds disagree with each other as well
@@ -92,22 +81,24 @@ def test_iou_vs_cpu_oracle_tolerance():
     np.testing.assert_allclose(ours, cpu, rtol=0, atol=1e-5)  # FMA contraction only
 
 
-@pytest.mark.parametrize("n,span,seed", [(1, 100, 0), (63, 200, 1), (64, 200, 2), (65, 200, 3), (1000, 300, 4),
-                                         (5000, 1024, 5), (30000, 1024, 6), (4097, 16384, 7)])
-def test_keep_bitexact_vs_reference_cuda_kernel(ref_ext, n, span, seed):
+@pytest.mark.parametrize("n,span,seed", KEEP_CASES)
+def test_keep_bitexact_vs_reference_cuda_kernel(n, span, seed):
     d, s, _ = rboxes(n, span, seed)
     ours = _nms(d, s, 0.4)
-    ref = ref_ext.nms_rotated_cuda(torch.from_numpy(d).to(DEV), torch.from_numpy(s).to(DEV), 0.4).cpu().numpy()
+    want = keep_from_bits(ref(f"keep/{n}_{span}_{seed}"), s)
     assert ours.dtype == np.int64
-    assert np.array_equal(ours, ref), f"n={n}: {len(ours)} vs {len(ref)} kept"
+    assert np.array_equal(ours, want), f"n={n}: {len(ours)} vs {len(want)} kept"
 
 
-@pytest.mark.parametrize("thr", [0.1, 0.2, 0.45, 0.7])
-def test_keep_thresholds_vs_reference_cuda_kernel(ref_ext, thr):
-    d, s, _ = rboxes(8000, 600, 21, n_classes=3)
+def threshold_case():
+    return rboxes(8000, 600, 21, n_classes=3)
+
+
+@pytest.mark.parametrize("thr", THRESHOLDS)
+def test_keep_thresholds_vs_reference_cuda_kernel(thr):
+    d, s, _ = threshold_case()
     ours = _nms(d, s, thr)
-    ref = ref_ext.nms_rotated_cuda(torch.from_numpy(d).to(DEV), torch.from_numpy(s).to(DEV), thr).cpu().numpy()
-    assert np.array_equal(ours, ref)
+    assert np.array_equal(ours, keep_from_bits(ref(f"thr/{thr}"), s))
     assert len(ours) < 8000  # something is suppressed
 
 
@@ -148,7 +139,7 @@ def test_ge_vs_gt_differ_on_exact_threshold():
     assert _nms(d, s, 1.0, strict_gt=False).tolist() == [0]
 
 
-def test_golden_fixtures(ref_ext):
+def test_golden_fixtures():
     g = np.load(ROOT / "tests" / "golden" / "nms_golden.npz")
     for k in sorted({x.split("/")[0] for x in g.files}):
         d, s, thr = g[f"{k}/dets"], g[f"{k}/scores"], float(g[f"{k}/thr"])
@@ -156,8 +147,7 @@ def test_golden_fixtures(ref_ext):
             # SURVEY 8(c) known-answer boxes: 2 and 3 are the same square written two ways, a degenerate
             # pair on which the reference's own CPU and CUDA arithmetic disagree (FMA contraction), so the
             # device result is pinned to the reference CUDA kernel, not to the CPU fixture
-            ref = ref_ext.nms_rotated_cuda(torch.from_numpy(d).to(DEV), torch.from_numpy(s).to(DEV), thr).cpu().numpy()
-            assert np.array_equal(_nms(d, s, thr, strict_gt=True), ref), k
+            assert np.array_equal(_nms(d, s, thr, strict_gt=True), keep_from_bits(ref(f"kat/{k}"), s)), k
             continue
         # fixtures hold the reference CPU extension's keep (>=, host hull); margin-checked at creation
         ours = _nms(d, s, thr, strict_gt=False)
@@ -231,26 +221,25 @@ def test_batched_equals_per_image():
     assert rc == 0 and (cnt.cpu().numpy() == -1).all()
 
 
-def test_batched_cluster_scan_equals_reference_kernel():
-    """Images with >= 40 960 boxes take the cluster form of the greedy scan (k_reduce_cluster: 8 CTAs per image sharing the
-    removed-set through distributed shared memory), smaller ones the single CTA - in the same batched call.  Checker: the
-    reference's own CUDA kernel K1 per image (oracle/_ref; the CPU oracle needs n x kept pair tests, minutes at this size),
-    with and without max_keep."""
-    from yolov5_obb_b200 import _lib
-    try:
-        from oracle.build_ref import load_ref
-        ref = load_ref()
-    except Exception:
-        pytest.skip("oracle/_ref (reference nms_rotated_cuda) not built")
-    L = _lib.lib()
+def cluster_case():
+    """Five images of 45 000, 0, 64, 5 000 and 41 000 boxes, their image ids in a seeded random order."""
     sizes = [45000, 0, 64, 5000, 41000]
-    B = len(sizes)
     parts = [rboxes(n, 1024, 60 + i) for i, n in enumerate(sizes)]
     d = np.concatenate([p[0] for p in parts])
     s = np.concatenate([p[1] for p in parts])
     img = np.concatenate([np.full(len(p[0]), i, np.int32) for i, p in enumerate(parts)])
     perm = np.random.default_rng(1).permutation(len(d))
-    d, s, img = d[perm], s[perm], img[perm]
+    return d[perm], s[perm], img[perm], len(sizes)
+
+
+def test_batched_cluster_scan_equals_reference_kernel():
+    """Images with >= 40 960 boxes take the cluster form of the greedy scan (k_reduce_cluster: 8 CTAs per image sharing the
+    removed-set through distributed shared memory), smaller ones the single CTA - in the same batched call.  Checker: the
+    reference's own CUDA kernel K1 per image (stored keep lists; the CPU oracle needs n x kept pair tests, minutes at this
+    size), with and without max_keep."""
+    from yolov5_obb_b200 import _lib
+    L = _lib.lib()
+    d, s, img, B = cluster_case()
     td, ts, ti = (torch.from_numpy(x).to(DEV) for x in (d, s, img))
     n = len(d)
     keep = torch.empty(n, dtype=torch.int64, device=DEV)
@@ -259,9 +248,8 @@ def test_batched_cluster_scan_equals_reference_kernel():
     ws = torch.empty(L.y5obb_nms_workspace_bytes(n, B, 45000), dtype=torch.uint8, device=DEV)
     exp = []
     for b in range(B):
-        idx = torch.from_numpy(np.flatnonzero(img == b)).to(DEV)
-        exp.append(idx[ref.nms_rotated_cuda(td[idx].contiguous(), ts[idx].contiguous(), 0.4)].cpu().numpy() if len(idx)
-                   else np.zeros(0, np.int64))
+        idx = np.flatnonzero(img == b)
+        exp.append(idx[keep_from_bits(ref(f"cluster/{b}"), s[idx])])
     for max_keep in (0, 700):
         rc = L.y5obb_nms_rotated_batched_f32(td.data_ptr(), ts.data_ptr(), ti.data_ptr(), n, B, 45000, 0.4, 1, max_keep,
                                              keep.data_ptr(), cnt.data_ptr(), off.data_ptr(), ws.data_ptr(), ws.numel(),

@@ -23,7 +23,11 @@ def test_mirror_init_and_oracle_forward_match_reference(size):
     pred, _ = model_ref.forward(m, x)
     ref = torch.from_numpy(G[f"{size}/pred"])
     assert pred.shape == ref.shape == (1, 3 * (8 * 12 + 4 * 6 + 2 * 3), 200)
-    assert (pred - ref).abs().max().item() < 1e-5
+    # 1e-5, or 16 float32 ulps of the value where that is more: the box columns reach ~400 px, where one ulp is 3e-5, and
+    # the CPU convolutions' summation order (thread count, instruction set) moves them by a few ulps - one thread instead
+    # of eight: up to 4.7 ulps; an fp64 forward differs from the stored fp32 output by up to 3
+    tol = (16 * torch.finfo(torch.float32).eps * ref.abs()).clamp_min(1e-5)
+    assert ((pred - ref).abs() < tol).all(), (pred - ref).abs().max().item()
 
 
 def test_model_structure_mirrors_reference():

@@ -1,15 +1,16 @@
-"""CPU tests: the oracle against the committed golden vectors and (where oracle/_ref is present)
-against the reference's own CPU extension compiled from /root/reference."""
+"""CPU tests: the oracle against the committed golden vectors, among them the keep lists of the reference's own CPU
+extension (tests/refgolden.py)."""
 from pathlib import Path
 
 import numpy as np
 import pytest
-import torch
 
 import oracle
 from tests.boxgen import rboxes, degenerate_pairs
+from tests.refgolden import keep_from_bits, ref
 
 ROOT = Path(__file__).resolve().parents[1]
+PIN_CASES = [(400, 250, 0.4, 0), (1500, 800, 0.3, 1), (900, 5000, 0.45, 2), (257, 100, 0.6, 3)]
 
 
 def test_oracle_matches_golden_keep_lists():
@@ -34,12 +35,11 @@ def test_oracle_matches_golden_iou_values():
     assert abs(v[0] - 1.0) < 1e-6 and v[1] == 0.0 and v[2] == 0.0 and abs(v[3] - 0.6) < 1e-6
 
 
-@pytest.mark.parametrize("n,span,thr,seed", [(400, 250, 0.4, 0), (1500, 800, 0.3, 1), (900, 5000, 0.45, 2),
-                                             (257, 100, 0.6, 3)])
-def test_oracle_pinned_to_reference_cpu_extension(ref_ext, n, span, thr, seed):
+@pytest.mark.parametrize("n,span,thr,seed", PIN_CASES)
+def test_oracle_pinned_to_reference_cpu_extension(n, span, thr, seed):
     d, s, _ = rboxes(n, span, seed, n_classes=4)
-    ref = ref_ext.nms_rotated_cpu(torch.from_numpy(d), torch.from_numpy(s), thr).numpy()
-    assert np.array_equal(oracle.nms_rotated(d, s, thr, mode=0), ref)
+    want = keep_from_bits(ref(f"cpu_keep/{n}_{span}_{thr}_{seed}"), s)
+    assert np.array_equal(oracle.nms_rotated(d, s, thr, mode=0), want)
 
 
 def test_obb_nms_wrapper_semantics():

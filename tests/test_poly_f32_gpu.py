@@ -1,7 +1,8 @@
 """GPU parity of the float polygon NMS / rotated-box overlaps (csrc/poly_f32.cu; SURVEY rows A14, B4) against the reference's
-own kernels, compiled unmodified from /root/reference/DOTA_devkit/poly_nms_gpu/*.cu for sm_100a into oracle/_ref
-(oracle/build_ref.build_polygpu): IoU matrices bit for bit, keep lists equal - through the devkit's host-pointer C ABI
-(`_poly_nms`, `_overlaps`), and through the device-pointer ops behind nms_rotated_ext.nms_poly."""
+own kernels, DOTA_devkit/poly_nms_gpu/*.cu compiled unmodified for sm_100a (oracle/build_ref.build_polygpu), whose outputs on
+the seeded inputs below are stored in tests/golden/ref_kernels_golden.npz (tests/refgolden.py): IoU matrices bit for bit, keep
+lists equal - through the devkit's host-pointer C ABI (`_poly_nms`, `_overlaps`), and through the device-pointer ops behind
+nms_rotated_ext.nms_poly."""
 import ctypes
 
 import numpy as np
@@ -10,17 +11,14 @@ import torch
 
 from tests.boxgen import rboxes
 from tests.polygen import merge_dets
+from tests.refgolden import assert_bit_equal, ref
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 
 
-def _ref():
-    try:
-        from oracle.build_ref import load_polygpu
-        return load_polygpu()
-    except FileNotFoundError:
-        pytest.skip("oracle/_ref/libref_polygpu_*.so not built")
+OVERLAP_CASES = ((0, 300, 257, 600.0), (1, 64, 1000, 200.0), (2, 1, 1, 50.0))
+POLY_NMS_CASES = [(1, 0, 0.3), (63, 1, 0.1), (64, 2, 0.3), (65, 3, 0.5), (3000, 4, 0.3), (5000, 5, 0.1)]
 
 
 def _rboxes5(n, span, seed, degenerate=True):
@@ -36,21 +34,23 @@ def _rboxes5(n, span, seed, degenerate=True):
     return d
 
 
+def overlap_inputs(seed, n, k, span):
+    b, q = _rboxes5(n, span, seed), _rboxes5(k, span, 100 + seed)
+    if n > 8 and k > 8:
+        q[:8] = b[:8]
+    return b, q
+
+
 def test_overlaps_bit_exact_host_abi_and_device_op():
-    _, ref_overlaps = _ref()
     from yolov5_obb_b200.devkit import poly_overlaps, poly_overlaps_device
-    for seed, n, k, span in ((0, 300, 257, 600.0), (1, 64, 1000, 200.0), (2, 1, 1, 50.0)):
-        b, q = _rboxes5(n, span, seed), _rboxes5(k, span, 100 + seed)
-        if n > 8 and k > 8:
-            q[:8] = b[:8]
-        want = np.zeros((n, k), np.float32)
-        ref_overlaps(want.ctypes.data, b.ctypes.data, q.ctypes.data, n, k, 0)
+    for seed, n, k, span in OVERLAP_CASES:
+        b, q = overlap_inputs(seed, n, k, span)
         got = poly_overlaps(b, q)
-        assert (want > 0.05).mean() > 0.01, "the case must contain overlapping pairs"
-        bad = np.flatnonzero(got.view(np.uint32).ravel() != want.view(np.uint32).ravel())
-        assert bad.size == 0, (seed, bad.size, got.ravel()[bad[:5]], want.ravel()[bad[:5]])
+        assert got.shape == (n, k)
+        assert_bit_equal(got, f"overlaps/{seed}")
+        assert (got > 0.05).mean() > 0.01, "the case must contain overlapping pairs"
         dev = poly_overlaps_device(torch.from_numpy(b).to(DEV), torch.from_numpy(q).to(DEV)).cpu().numpy()
-        assert np.array_equal(dev.view(np.uint32), want.view(np.uint32))
+        assert np.array_equal(dev.view(np.uint32), got.view(np.uint32))
 
 
 def _sorted_dets(n, seed):
@@ -58,23 +58,19 @@ def _sorted_dets(n, seed):
     return np.ascontiguousarray(d[np.argsort(-d[:, 8], kind="stable")])
 
 
-@pytest.mark.parametrize("n,seed,thr", [(1, 0, 0.3), (63, 1, 0.1), (64, 2, 0.3), (65, 3, 0.5), (3000, 4, 0.3), (5000, 5, 0.1)])
+@pytest.mark.parametrize("n,seed,thr", POLY_NMS_CASES)
 def test_poly_nms_keep_lists_equal_reference(n, seed, thr):
-    ref_poly_nms, _ = _ref()
     from yolov5_obb_b200 import _lib
     from yolov5_obb_b200.devkit import poly_gpu_nms
     from yolov5_obb_b200.nms_rotated import nms_poly, poly_nms
     d = _sorted_dets(n, seed)
-    keep = np.zeros(n, np.int32)
-    num = ctypes.c_int(0)
-    ref_poly_nms(keep.ctypes.data, ctypes.addressof(num), d.ctypes.data, n, 9, thr, 0)
-    want = keep[:num.value].copy()
+    want = ref(f"poly_nms/{n}_{seed}_{thr}")
     assert n < 100 or 0 < len(want) < n
     # (1) the devkit's host-pointer C ABI (K3 contract: the caller's order is the processing order)
     got = np.zeros(n, np.int32)
     gnum = ctypes.c_int(0)
     _lib.lib().y5obb_devkit_poly_nms(got.ctypes.data, ctypes.addressof(gnum), d.ctypes.data, n, 9, thr, 0)
-    assert gnum.value == num.value and np.array_equal(got[:gnum.value], want)
+    assert gnum.value == len(want) and np.array_equal(got[:gnum.value], want)
     # (2) the .pyx-level function on UNSORTED input (host argsort as the .pyx) and (3) the device op behind nms_poly (K2): both
     # return indices into the caller's order
     perm = np.random.default_rng(seed).permutation(n)
