@@ -24,7 +24,7 @@ extern "C" {
 #define Y5OBB_EARCH 4      /* device is not sm_100 */
 
 /* ---- library ------------------------------------------------------------------------------- */
-int y5obb_abi_version(void);            /* bumps when a signature changes */
+int y5obb_abi_version(void);            /* bumps when a signature, an entry point or a flag is changed or removed */
 int y5obb_last_cuda_error(void);        /* cudaError_t of the last failing CUDA call on this thread */
 const char* y5obb_build_info(void);     /* "sm_100a nvcc <ver> <date>" */
 
@@ -112,22 +112,14 @@ typedef struct y5obb_conv y5obb_conv_t;
 #define Y5OBB_CONV_MODE_CONV 0    /* bf16 NHWC output (+ optional residual / 2x up-sampled copy) */
 #define Y5OBB_CONV_MODE_DETECT 1  /* Detect head: fp32 [B, rows, no] output, optional sigmoid+decode */
 
+/* flags: any bit not defined here makes y5obb_conv_create return Y5OBB_EINVAL */
 #define Y5OBB_CONV_NO_ROWSHIFT 1   /* flags: force one TMA load per tap (debug / A-B comparison) */
 #define Y5OBB_CONV_NO_RESIDENT 2   /* flags: always stream the weight tiles */
 #define Y5OBB_CONV_BIAS_HALVED 8    /* flags: REQUIRED when act = 1: `bias` holds 0.5 * b (SiLU is evaluated as h + h*tanh(h), h = x/2) */
-#define Y5OBB_CONV_NO_GROUP 16      /* flags: one (tap, K-chunk) unit per pipeline stage */
 #define Y5OBB_CONV_NO_PAIRW 4      /* flags: stride-2 convs use TMA element strides along W instead of the pixel-pair view */
-#define Y5OBB_CONV_NO_PDL 32       /* flags: plain stream-ordered launch (default: programmatic dependent launch - the kernel's
-                                      prologue overlaps the previous kernel's tail and it waits, griddepcontrol.wait, before its
-                                      first global-memory access; also switched off by the environment variable Y5OBB_NO_PDL=1) */
-#define Y5OBB_CONV_MSUB1 128       /* flags: 128-pixel tiles only (default: up to four 128-pixel sub-tiles per tile) */
 #define Y5OBB_CONV_NO_UP_TMA 2048  /* flags: the 2x up-sampled copy through per-thread stores (default: four TMA stores of the staged tile) */
-#define Y5OBB_CONV_NO_DUAL 4096    /* flags: always one CTA per SM.  (Two CTAs per SM - 256 TMEM columns, half the shared memory and four
-                                      epilogue warps each - is an opt-in experiment, environment variable Y5OBB_DUAL; measured slower) */
 #define Y5OBB_CONV_NO_RES_RED 16384 /* flags: when `res` IS `out` (in-place Bottleneck add) the default adds the tile into memory with a TMA
                                       reduce-add (bf16 add at L2: the sum is rounded twice); this flag keeps the epilogue's own fp32 add */
-#define Y5OBB_CONV_EPI2 8192       /* flags: reserved (two staging buffers per epilogue warp are the default; four: environment variable Y5OBB_EPI_BUFS=4, measured slower) */
-#define Y5OBB_CONV_ACC2 64         /* flags: two TMEM accumulator stages only (A-B comparison; default: as many as 512 columns hold) */
 
 typedef struct {
   const void* in;            /* bf16 NHWC slice */
@@ -172,10 +164,6 @@ void y5obb_conv_destroy(y5obb_conv_t* conv);
 /* Profiling aid: CTA 0 of every later run writes clock64() stamps of its producer / MMA / epilogue roles for its first 32
  * tiles into dev_buf ([3][32][8] uint64, device memory; NULL switches it off).  Results are unaffected. */
 int y5obb_conv_debug_timestamps(y5obb_conv_t* conv, unsigned long long* dev_buf);
-/* Profiling aid: resident CTAs per SM the runtime grants the one-CTA (dual = 0, 320 threads) or two-CTA (dual = 1, 192 threads)
- * instantiation of the kernel for a given dynamic shared-memory size, with its register count and static shared memory. */
-int y5obb_conv_debug_occupancy(int dual, int threads, size_t dyn_smem, int* blocks_per_sm, int* regs, int* static_smem);
-int y5obb_wgrad_debug_occupancy(size_t dyn_smem, int* blocks_per_sm, int* regs);
 
 /* ---- HBM-bound helpers around the conv stack -------------------------------------------------
  * y5obb_stem_s2d: NCHW fp32 image [B,3,H,W] -> 2x2 space-to-depth NHWC bf16 [B,H/2,W/2,16] (channel

@@ -30,9 +30,26 @@ def test_python_prototypes_cover_the_abi():
     from yolov5_obb_b200 import _lib
     assert set(_lib.PROTOTYPES) == _declared()
     L = _lib.lib()
-    assert L.y5obb_abi_version() >= 1
+    assert L.y5obb_abi_version() >= 2
     assert b"sm_100a" in L.y5obb_build_info()
     assert L.y5obb_nms_workspace_bytes(1000, 1, 1000) > 1000 * 24
+
+
+def test_conv_create_rejects_unknown_flags():
+    """A flags bit y5obb.h does not define (a retired option such as 128, or 256-1024) is refused before any CUDA call, rather
+    than silently giving a different kernel.  Nothing is dereferenced during create, so fake aligned device addresses do."""
+    from yolov5_obb_b200 import _lib
+    from yolov5_obb_b200.conv import ConvDesc
+    d = ConvDesc()
+    d.in_, d.in_pix_stride, d.B, d.Hin, d.Win, d.Cin = 0x10000, 16, 1, 8, 8, 16
+    d.w, d.bias = 0x20000, 0x30000
+    d.Cout, d.KH, d.KW, d.stride = 16, 1, 1, 1
+    d.out, d.out_pix_stride = 0x40000, 16
+    h = ctypes.c_void_p()
+    for flags in (256, 128):
+        d.flags = flags
+        assert _lib.lib().y5obb_conv_create(ctypes.byref(d), ctypes.byref(h)) == 1, flags  # Y5OBB_EINVAL
+    assert not h.value
 
 
 def test_no_product_import_of_oracle():

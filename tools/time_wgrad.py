@@ -1,5 +1,5 @@
-"""Stand-alone timing of the wgrad kernel on training-sized layers (debug aid).  Y5OBB_WGRAD_DBG=1|2 skips TMA|MMA."""
-import os, sys, torch
+"""Stand-alone timing of the wgrad kernel on training-sized layers (debug aid)."""
+import sys, torch
 from yolov5_obb_b200.train_ops import Wgrad
 DEV = "cuda:0"
 CASES = [(8, 48, 48, 256, 256, 3, 1), (8, 96, 96, 128, 128, 3, 1), (8, 48, 96, 512, 512, 3, 2), (8, 192, 192, 64, 64, 3, 1),
@@ -22,4 +22,4 @@ for (B, Cin, Cout, H, W, k, s) in [CASES[i] for i in sel]:
     torch.cuda.synchronize()
     us = e0.elapsed_time(e1) * 100
     fl = 2.0 * B * Ho * Wo * Cout * Cin * k * k
-    print(f"dbg={os.environ.get('Y5OBB_WGRAD_DBG', '0')} {Cin}->{Cout} k{k} s{s} {Ho}x{Wo}: {us:7.1f} us  {fl / us / 1e6:6.1f} TF/s", flush=True)
+    print(f"{Cin}->{Cout} k{k} s{s} {Ho}x{Wo}: {us:7.1f} us  {fl / us / 1e6:6.1f} TF/s", flush=True)

@@ -41,8 +41,6 @@ PROTOTYPES = {
                         + [ctypes.POINTER(c_int)] * 4),
     "y5obb_conv_destroy": (None, [c_void_p]),
     "y5obb_conv_debug_timestamps": (c_int, [c_void_p, c_void_p]),
-    "y5obb_wgrad_debug_occupancy": (c_int, [c_size_t] + [ctypes.POINTER(c_int)] * 2),
-    "y5obb_conv_debug_occupancy": (c_int, [c_int, c_int, c_size_t] + [ctypes.POINTER(c_int)] * 3),
     "y5obb_loss_workspace_bytes": (c_size_t, [c_void_p]),
     "y5obb_loss_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "y5obb_loss_backward": (c_int, [c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),

@@ -14,8 +14,8 @@
 //             stride-2 convs use the tensor map's element strides.
 //   W tile  = 2-D TMA box {BK, BN} of weights packed [tap][Cout_pad][Cin_pad] (K-major).
 //   Both land in 32/64/128-byte swizzled K-major layouts that tcgen05.mma consumes directly.
-// One persistent CTA per SM, 6 warps: TMA producer, MMA issuer (+TMEM owner), 4 epilogue warps;
-// two TMEM accumulators so the epilogue of tile i overlaps the MMAs of tile i+1.
+// One persistent CTA per SM, 10 warps: TMA producer, MMA issuer (+TMEM owner), 8 epilogue warps;
+// up to 8 TMEM accumulator stages so the epilogue of tile i overlaps the MMAs of the tiles after it.
 //
 // Roofline: tensor pipe for the wide layers (2*128*BN*K flop per tile), HBM for the narrow ones
 // (algorithmic bytes = input pixels*Cin*2 + output pixels*Cout*2 [+ residual] per image).
@@ -36,11 +36,15 @@ namespace {
 constexpr int BM = 128;  // output pixels per tile == TMEM lanes
 constexpr int MAX_STAGES = 16;
 constexpr int MAX_ACC = 8;                // TMEM accumulator stages: 512 columns / accumulator stride
-constexpr int NUM_THREADS = 320;          // TMA producer, MMA issuer, 8 epilogue warps (the one-CTA-per-SM configuration)
-constexpr int EPI_WARPS = 8;              // ... or 4 epilogue warps (192 threads) when two CTAs share an SM, see ConvK::epi_warps
+constexpr int NUM_THREADS = 320;          // TMA producer, MMA issuer, 8 epilogue warps
+constexpr int EPI_WARPS = 8;
+constexpr int TMEM_COLS = 512;            // the CTA owns all of the SM's tensor memory
+// Staging buffers per epilogue warp, used alternately: in-kernel stamps show ~100 cycles between "accumulator loaded" and
+// "staging buffer free" with two, i.e. the TMA stores are not what the epilogue waits for (four measured slower: they cost
+// operand-ring depth)
+constexpr int EPI_BUFS = 2;
 constexpr int EPI_STAGE_CONV = 32 * 64;    // 32 pixels x 32 bf16 channels, 64-byte swizzled
 constexpr int EPI_STAGE_DET = 32 * 128;    // 32 pixels x 32 fp32 outputs, 128-byte swizzled
-constexpr int DUAL_SMEM = 110 * 1024;     // per CTA when two share an SM (228 KB per SM, 1 KB reserved per CTA)
 constexpr int SMEM_TOTAL = 224 * 1024;    // dynamic shared memory we ask for at most (227 KB is the hardware cap)
 
 enum Mode : int { MODE_CONV = 0, MODE_DETECT = 1 };
@@ -81,22 +85,11 @@ struct ConvK {
                        // [m * sub_cols, ...), A rows [m * 128, (m + 1) * 128) of the stage)
   int sub_cols;        // TMEM columns per sub-tile accumulator (acc_stride = m_sub * sub_cols)
   uint32_t a_sub16;    // (128 rows * row bytes) >> 4: descriptor distance between the sub-tiles' A rows
-  int pdl;             // launched with programmatic stream serialisation: griddepcontrol.wait before the first global access
-  int dbg;             // timing experiments only (results are garbage): 1 = no TMA loads, 2 = no MMAs, 4 = no epilogue work
   int pairw;           // 1: stride-2 conv whose input is viewed as horizontal pixel PAIRS (2*pix_stride channels per
                        // position): the column phase of a tap is a channel offset, so TMA reads contiguous rows
   int in_pix_stride;
-  int epi_warps;       // 8: one CTA per SM (all 512 TMEM columns, two epilogue groups); 4: TWO CTAs per SM, each with 256 TMEM
-                       // columns, half the shared memory and one epilogue group - two independent producer / MMA / epilogue
-                       // pipelines whose hand-shake bubbles overlap (ncu: no unit of the single pipeline is above 45 % busy)
-  int tmem_cols;       // 512 or 256
   int res_red;         // 1: the residual IS the output buffer (in-place Bottleneck add) and the tile leaves as a TMA reduce-add: no
                        // residual loads in the epilogue (the kernel then runs its no-residual flavour)
-  int res_prefetch;    // 1: the epilogue requests its next tile's residual lines into L2 (opt-in: Y5OBB_RES_PREFETCH=1; measured neutral)
-  int no_full_fence;   // 1: no tcgen05.fence::after_thread_sync after the operand-ring wait (A-B)
-  int mma_loop;        // 1: the MMA issuer uses the compact runtime loop for every unit shape (A-B against the unrolled sequences)
-  int wait_suspend;    // 1: the epilogue warps' wait on the accumulator uses the suspend-hint form of mbarrier.try_wait
-  int epi_bufs;        // staging buffers per epilogue warp (2 or 4): a buffer is reused only after its TMA store has read it
   int epi_tile_split;  // 1: epilogue warp group g handles the tiles whose accumulator is g (all columns); 0: both
                        // groups work on every tile and split its columns (few tiles per CTA)
   int rowshift;    // 1: one A stage holds Ht + KH - 1 image rows; the KH taps of a column read it at row offsets
@@ -219,7 +212,7 @@ __device__ __forceinline__ void mma_role(const ConvK& p, const MmaCtx& x) {
   const uint32_t a_bytes16 = p.a_bytes >> 4, a_sub16 = p.a_sub16, idesc = p.idesc, hi = x.hi;
   const int n_units = p.n_units, group = p.group, kchunks = p.kchunks, m_sub = p.m_sub, sub_cols = p.sub_cols, stages = p.stages;
   const int nk_last = ((p.Cin - (kchunks - 1) * p.BK) + 15) >> 4;  // MMAs per tap of the last (possibly ragged) K chunk
-  const bool resident = p.b_resident != 0, no_mma = (p.dbg & 2) != 0;
+  const bool resident = p.b_resident != 0;
   int s = 0, it = 0;
   uint32_t ph = 0, s_lo = x.ring_lo;
   for (int t = blockIdx.x; t < x.total_tiles; t += gridDim.x, ++it) {
@@ -235,29 +228,26 @@ __device__ __forceinline__ void mma_role(const ConvK& p, const MmaCtx& x) {
     for (int u0 = 0; u0 < n_units; u0 += group) {
       const int ng = min(group, n_units - u0);
       ptx::mbar_wait(&x.full_bar[s], ph);
-      // (no tcgen05.fence here: the operands were written by TMA, whose completion this mbarrier phase is; the fence is for
-      // ordering against other threads' tcgen05 operations - the accumulator hand-back above)
-      if (!p.no_full_fence) ptx::tc_fence_after();
+      // tcgen05.fence::after_thread_sync orders the MMAs below after this wait (leaving it out measured no faster)
+      ptx::tc_fence_after();
       if (u0 == 0) Y5_TS(1, it, 2);
       uint32_t a_lo = s_lo;
       for (int g = 0; g < ng; ++g) {
         const uint32_t b_lo = resident ? bres_lo : a_lo + a_bytes16;
         const bool last = kc + 1 == kchunks;
-        if (!no_mma) {
-          if (NK > 0 && (!last || nk_last == NK)) {
-            for (int m = 0; m < m_sub; ++m)  // the m_sub sub-tiles of the tile share this unit's weights
-              issue_unit_lo<KSUB, NK>(d_tmem + (uint32_t)(m * sub_cols), a_lo + (uint32_t)m * a_sub16, b_lo, hi, a_step, b_step, idesc, accumulate);
-          } else {
-            const int nk = last ? nk_last : (p.BK >> 4);
-            for (int m = 0; m < m_sub; ++m) {
-              uint32_t acc_m = accumulate;
-              for (int u = 0; u < x.ksub; ++u)
-                for (int j = 0; j < nk; ++j) {
-                  ptx::umma_bf16(d_tmem + (uint32_t)(m * sub_cols), desc_from(a_lo + (uint32_t)m * a_sub16 + (uint32_t)u * a_step + 2u * j, hi),
-                                 desc_from(b_lo + (uint32_t)u * b_step + 2u * j, hi), idesc, acc_m);
-                  acc_m = 1u;
-                }
-            }
+        if (NK > 0 && (!last || nk_last == NK)) {
+          for (int m = 0; m < m_sub; ++m)  // the m_sub sub-tiles of the tile share this unit's weights
+            issue_unit_lo<KSUB, NK>(d_tmem + (uint32_t)(m * sub_cols), a_lo + (uint32_t)m * a_sub16, b_lo, hi, a_step, b_step, idesc, accumulate);
+        } else {
+          const int nk = last ? nk_last : (p.BK >> 4);
+          for (int m = 0; m < m_sub; ++m) {
+            uint32_t acc_m = accumulate;
+            for (int u = 0; u < x.ksub; ++u)
+              for (int j = 0; j < nk; ++j) {
+                ptx::umma_bf16(d_tmem + (uint32_t)(m * sub_cols), desc_from(a_lo + (uint32_t)m * a_sub16 + (uint32_t)u * a_step + 2u * j, hi),
+                               desc_from(b_lo + (uint32_t)u * b_step + 2u * j, hi), idesc, acc_m);
+                acc_m = 1u;
+              }
           }
         }
         accumulate = 1u;
@@ -298,7 +288,6 @@ struct EpiTile {
   const CUtensorMap* tmu;  // up-sampled copy by TMA (null: per-thread stores through urow)
   int ubh;                 // cb * Hout + chh
   unsigned long long* ts;  // debug stamps of this tile's first chunk (slots 4..6 of the epilogue row) or null
-  int nbuf;                // staging buffers of this warp (2 or 4)
   bool red;                // the staged tile is ADDED to the destination (in-place residual) instead of stored
 };
 
@@ -327,10 +316,7 @@ __device__ __forceinline__ void conv_epi_tile(const EpiTile& e, int& sbuf, uint4
     ptx::tmem_ld_wait();
     if (e.ts && c0 == e.col_first) e.ts[5] = clock64();
     // the staging buffer about to be overwritten must have been read by its TMA store
-    if (e.leader) {
-      if (e.nbuf == 4) ptx::tma_store_wait_read<3>();
-      else ptx::tma_store_wait_read<1>();
-    }
+    if (e.leader) ptx::tma_store_wait_read<1>();
     __syncwarp();
     uint8_t* sb = e.stage + sbuf * e.stage_bytes + e.lane * 64;
 #pragma unroll
@@ -388,7 +374,7 @@ __device__ __forceinline__ void conv_epi_tile(const EpiTile& e, int& sbuf, uint4
       }
       ptx::tma_store_commit();
     }
-    sbuf = (sbuf + 1) & (e.nbuf - 1);
+    sbuf ^= 1;
   }
 }
 
@@ -398,7 +384,7 @@ struct EpiCtx {
   uint8_t* stage;    // this warp's staging buffers
   uint32_t bias_s;   // shared-memory address of the layer's bias
   int lane, e, q, half, hl, wl, box_w0, box_h0, col_first, col_step, total_tiles;
-  bool leader, one_group;
+  bool leader;
 };
 
 // The MODE_CONV epilogue's whole tile loop, specialised on the layer flavour (activation, residual, 2x up-sampled copy): the
@@ -419,17 +405,16 @@ __device__ __forceinline__ void epi_role_conv(const ConvK& p, const EpiCtx& x) {
   et.col_step = x.col_step;
   et.tm = &p.tmO;
   et.tmu = (UP && p.up_tma) ? &p.tmU : nullptr;
-  et.nbuf = p.epi_bufs;
   et.red = p.res_red != 0;
   const long long rstep = (long long)p.Ht * p.res_row_stride;                                 // residual: one sub-tile down
   const long long ustep = (long long)(2 * p.Ht) * (2 * p.Wout) * p.out2x_pix_stride;           // up-sampled copy: one sub-tile down
   const uint32_t lane_quarter = (uint32_t)(x.q * 32) << 16;
   for (int t = blockIdx.x; t < x.total_tiles; t += gridDim.x, ++it) {
     const int acc = it & (p.n_acc - 1);
-    if (p.epi_tile_split && !x.one_group && (it & 1) != x.half) continue;  // the other warp group owns this tile
+    if (p.epi_tile_split && (it & 1) != x.half) continue;  // the other warp group owns this tile
     const TileCoord c = decode_tile(p, t);
     const uint32_t acc_ph = (uint32_t)(it >> p.acc_shift) & 1u;
-    const bool ts_on = x.leader && (x.e & 3) == 0 && (p.epi_tile_split || x.one_group || x.e == 0);
+    const bool ts_on = x.leader && (x.e & 3) == 0 && (p.epi_tile_split || x.e == 0);
     const int h0 = c.h0 + x.hl, w = c.w0 + x.wl;
     const bool wvalid = w < p.Wout;
     const int nvalid = min(p.BN, p.Cout - c.n0);
@@ -448,50 +433,28 @@ __device__ __forceinline__ void epi_role_conv(const ConvK& p, const EpiCtx& x) {
       for (int g = 0; g < 4; ++g)
         rvn[g] = (r0 && x.col_first + g * 8 < nvalid) ? *reinterpret_cast<const uint4*>(r0 + x.col_first + g * 8) : make_uint4(0, 0, 0, 0);
     }
-    if (RES && p.res_prefetch) {
-      // The residual of the early layers comes from HBM (it left L2 two layers ago) and is fetched by the epilogue threads
-      // themselves, 64 bytes per thread and chunk, one chunk ahead: too few bytes in flight for a 2-3 k cycle latency.  So the
-      // lines this thread will need in its NEXT tile are requested into L2 now, a whole tile time ahead (no registers, no
-      // shared memory); the loads above then see an L2 hit.
-      const int tn = t + (int)gridDim.x * ((p.epi_tile_split && !x.one_group) ? 2 : 1);
-      if (tn < x.total_tiles) {
-        const TileCoord cn = decode_tile(p, tn);
-        const int hn = cn.h0 + x.hl, wn = cn.w0 + x.wl;
-        if (wn < p.Wout) {
-          const __nv_bfloat16* rn =
-              p.res + (long long)cn.b * p.res_img_stride + (long long)hn * p.res_row_stride + (long long)wn * p.res_pix_stride + cn.n0;
-          const int nvn = min(p.BN, p.Cout - cn.n0);
-          for (int m = 0; m < p.m_sub; ++m)
-            if (hn + m * p.Ht < p.Hout)
-              for (int c0 = x.col_first; c0 < nvn; c0 += x.col_step) ptx::prefetch_l2(rn + m * rstep + c0);
-        }
-      }
-    }
     et.bias = x.bias_s + (uint32_t)c.n0 * 4u;
     et.nvalid = nvalid;
     et.cn0 = c.n0;
     et.cw = c.w0 + x.box_w0;
     et.cb = c.b;
     if (ts_on) Y5_TS(2, it, 0);
-    if (p.wait_suspend) ptx::mbar_wait_suspend(&x.tmem_full[acc], acc_ph);
-    else ptx::mbar_wait(&x.tmem_full[acc], acc_ph);
+    ptx::mbar_wait_suspend(&x.tmem_full[acc], acc_ph);
     ptx::tc_fence_after();
     if (ts_on) Y5_TS(2, it, 1);
-    if (!(p.dbg & 4)) {
-      uint32_t taddr = x.tmem_base + (uint32_t)(acc * p.acc_stride) + lane_quarter;
-      int chh = c.h0 + x.box_h0;
-      for (int m = 0; m < p.m_sub; ++m) {  // the tile's 128-pixel sub-tiles, stacked along H
-        et.taddr = taddr;
-        et.chh = chh;
-        et.ubh = c.b * p.Hout + chh;
-        et.rrow = res_row(m);
-        et.rrow_next = res_row(m + 1);
-        et.urow = (UP && !et.tmu && wvalid && h0 + m * p.Ht < p.Hout) ? ubase + m * ustep : nullptr;
-        et.ts = (ts_on && m == 0 && p.ts && (int)blockIdx.x == p.ts_cta) ? p.ts + (2 * 32 + (it & 31)) * 8 : nullptr;
-        conv_epi_tile<ACT, RES, UP>(et, sbuf, rvn);
-        taddr += (uint32_t)p.sub_cols;
-        chh += p.Ht;
-      }
+    uint32_t taddr = x.tmem_base + (uint32_t)(acc * p.acc_stride) + lane_quarter;
+    int chh = c.h0 + x.box_h0;
+    for (int m = 0; m < p.m_sub; ++m) {  // the tile's 128-pixel sub-tiles, stacked along H
+      et.taddr = taddr;
+      et.chh = chh;
+      et.ubh = c.b * p.Hout + chh;
+      et.rrow = res_row(m);
+      et.rrow_next = res_row(m + 1);
+      et.urow = (UP && !et.tmu && wvalid && h0 + m * p.Ht < p.Hout) ? ubase + m * ustep : nullptr;
+      et.ts = (ts_on && m == 0 && p.ts && (int)blockIdx.x == p.ts_cta) ? p.ts + (2 * 32 + (it & 31)) * 8 : nullptr;
+      conv_epi_tile<ACT, RES, UP>(et, sbuf, rvn);
+      taddr += (uint32_t)p.sub_cols;
+      chh += p.Ht;
     }
     if (ts_on) Y5_TS(2, it, 2);
     ptx::tc_fence_before();
@@ -500,11 +463,7 @@ __device__ __forceinline__ void epi_role_conv(const ConvK& p, const EpiCtx& x) {
   }
 }
 
-// DUAL = false: 320 threads, one CTA per SM.  DUAL = true: launched with 192 threads (producer, MMA issuer, four epilogue
-// warps), two CTAs per SM: 6 warps are allocated as 8, so 2 x 8 x 32 x 120 registers = 61 440 of the SM's 65 536 (at 128
-// registers the runtime grants one CTA only, profiles/r2_occupancy.txt).
-template <bool DUAL>
-__global__ void __launch_bounds__(DUAL ? 192 : NUM_THREADS) __maxnreg__(DUAL ? 120 : 168) conv_tc_kernel(const __grid_constant__ ConvK p) {
+__global__ void __launch_bounds__(NUM_THREADS) conv_tc_kernel(const __grid_constant__ ConvK p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t full_bar[MAX_STAGES];
   __shared__ __align__(8) uint64_t empty_bar[MAX_STAGES];
@@ -535,13 +494,13 @@ __global__ void __launch_bounds__(DUAL ? 192 : NUM_THREADS) __maxnreg__(DUAL ? 1
     }
     for (int a = 0; a < p.n_acc; ++a) {
       ptx::mbar_init(&tmem_full[a], 1);
-      ptx::mbar_init(&tmem_empty[a], (p.epi_tile_split || p.epi_warps == 4) ? 128 : EPI_WARPS * 32);
+      ptx::mbar_init(&tmem_empty[a], p.epi_tile_split ? 128 : EPI_WARPS * 32);
     }
     ptx::mbar_init(&wres_bar, 1);
     ptx::fence_mbar_init();
   }
   if (warp == 1) {
-    ptx::tmem_alloc(&tmem_base_smem, (uint32_t)p.tmem_cols);
+    ptx::tmem_alloc(&tmem_base_smem, (uint32_t)TMEM_COLS);
     ptx::tmem_relinquish();
   }
   ptx::tc_fence_before();
@@ -551,10 +510,8 @@ __global__ void __launch_bounds__(DUAL ? 192 : NUM_THREADS) __maxnreg__(DUAL ? 1
   // Programmatic dependent launch: everything above (barriers, TMEM, descriptor prefetch) overlapped the previous kernel's
   // tail; from here on global memory is touched, so the previous grid must have completed and flushed.  Only then may the
   // NEXT kernel start its own prologue (its pre-wait phase never touches memory, and it finds kernel N-1's inputs final).
-  if (p.pdl) {
-    ptx::griddep_wait();
-    ptx::griddep_launch_dependents();
-  }
+  ptx::griddep_wait();
+  ptx::griddep_launch_dependents();
 
   if (warp == 0) {
     // ===================== TMA producer =====================
@@ -582,11 +539,7 @@ __global__ void __launch_bounds__(DUAL ? 192 : NUM_THREADS) __maxnreg__(DUAL ? 1
           ptx::mbar_wait(&empty_bar[s], ph ^ 1u);
           if (u0 == 0) Y5_TS(0, pit, 1);
           uint8_t* sbase = smem + (size_t)s * stage_bytes;
-          if (p.dbg & 1) {
-            ptx::mbar_arrive(&full_bar[s]);
-          } else {
-            ptx::mbar_expect_tx(&full_bar[s], unit_tx * (uint32_t)ng);
-          }
+          ptx::mbar_expect_tx(&full_bar[s], unit_tx * (uint32_t)ng);
           for (int g = 0; g < ng; ++g) {
             int wi = c.w0 * p.stride + kw - p.pad_w;
             const int hi = c.h0 * p.stride + kh - p.pad_h;
@@ -597,15 +550,13 @@ __global__ void __launch_bounds__(DUAL ? 192 : NUM_THREADS) __maxnreg__(DUAL ? 1
               wi = c.w0 + ((off - phase) >> 1);
               cbase = phase * p.in_pix_stride;
             }
-            if (!(p.dbg & 1)) {
-              uint8_t* sa = sbase + (size_t)g * unit_bytes;
-              uint8_t* sb = sa + p.a_bytes;
-              ptx::tma_load_4d(sa, &p.tmA, &full_bar[s], cbase + kc * p.BK, wi, hi, c.b);
-              for (int j = 0; j < p.b_per_stage; ++j) {
-                const int tap = (p.rowshift ? j : kh) * p.KW + kw;
-                ptx::tma_load_2d(sb + (size_t)j * p.b_stage_bytes, &p.tmB, &full_bar[s], kc * p.BK,
-                                 tap * p.cout_pad + c.n0);
-              }
+            uint8_t* sa = sbase + (size_t)g * unit_bytes;
+            uint8_t* sb = sa + p.a_bytes;
+            ptx::tma_load_4d(sa, &p.tmA, &full_bar[s], cbase + kc * p.BK, wi, hi, c.b);
+            for (int j = 0; j < p.b_per_stage; ++j) {
+              const int tap = (p.rowshift ? j : kh) * p.KW + kw;
+              ptx::tma_load_2d(sb + (size_t)j * p.b_stage_bytes, &p.tmB, &full_bar[s], kc * p.BK,
+                               tap * p.cout_pad + c.n0);
             }
             if (++kc == p.kchunks) {
               kc = 0;
@@ -646,9 +597,7 @@ __global__ void __launch_bounds__(DUAL ? 192 : NUM_THREADS) __maxnreg__(DUAL ? 1
       x.total_tiles = total_tiles;
       x.ksub = ksub;
       const int nkf = (min(p.BK, p.Cin) + 15) >> 4;  // MMAs per tap of a full K chunk
-      if (p.mma_loop) {
-        mma_role<0, 0>(p, x);
-      } else if (ksub == 3) {
+      if (ksub == 3) {
         switch (nkf) {
           case 1: mma_role<3, 1>(p, x); break;
           case 2: mma_role<3, 2>(p, x); break;
@@ -680,18 +629,17 @@ __global__ void __launch_bounds__(DUAL ? 192 : NUM_THREADS) __maxnreg__(DUAL ? 1
     // this warp's 32 pixels as a TMA box: {32 ch, bw, 32 / bw, 1}
     const int bw = min(p.Wt, 32);
     const int box_h0 = (q * 32) / p.Wt, box_w0 = (q * 32) % p.Wt;
-    uint8_t* stage = smem + (size_t)p.stages * stage_bytes + (size_t)e * ((size_t)p.epi_bufs * p.epi_stage_bytes);
+    uint8_t* stage = smem + (size_t)p.stages * stage_bytes + (size_t)e * ((size_t)EPI_BUFS * p.epi_stage_bytes);
     // the layer's bias in shared memory: with 224 KB of the SM configured as shared memory the L1 that is left is a few KB, the
     // residual stream evicts the bias line at every chunk and each 32-column chunk then waited an L2 round trip (~700+ cycles
     // in the in-kernel stamps) for the SAME 128 bytes
-    float* bias_s = reinterpret_cast<float*>(smem + (size_t)p.stages * stage_bytes + (size_t)p.epi_warps * p.epi_bufs * p.epi_stage_bytes);
-    for (int i = (int)threadIdx.x - 64; i < p.cout_pad + 32; i += 32 * p.epi_warps) bias_s[i] = __ldg(p.bias + i);
-    asm volatile("bar.sync 1, %0;" ::"r"(32 * p.epi_warps) : "memory");
+    float* bias_s = reinterpret_cast<float*>(smem + (size_t)p.stages * stage_bytes + (size_t)EPI_WARPS * EPI_BUFS * p.epi_stage_bytes);
+    for (int i = (int)threadIdx.x - 64; i < p.cout_pad + 32; i += 32 * EPI_WARPS) bias_s[i] = __ldg(p.bias + i);
+    asm volatile("bar.sync 1, %0;" ::"r"(32 * EPI_WARPS) : "memory");
     int sbuf = 0;
     int it = 0;
-    const bool one_group = p.epi_warps == 4;                              // a single epilogue group takes every tile, every column
-    const int col_first = (p.epi_tile_split || one_group) ? 0 : half * 32;  // first 32-column chunk of this warp
-    const int col_step = (p.epi_tile_split || one_group) ? 32 : 64;
+    const int col_first = p.epi_tile_split ? 0 : half * 32;  // first 32-column chunk of this warp
+    const int col_step = p.epi_tile_split ? 32 : 64;
     if (p.mode == MODE_CONV) {  // one specialised instantiation of the whole loop per layer flavour
       EpiCtx x;
       x.tmem_full = tmem_full;
@@ -711,7 +659,6 @@ __global__ void __launch_bounds__(DUAL ? 192 : NUM_THREADS) __maxnreg__(DUAL ? 1
       x.col_step = col_step;
       x.total_tiles = total_tiles;
       x.leader = leader;
-      x.one_group = one_group;
       const int flavour = (p.act ? 1 : 0) | ((p.res && !p.res_red) ? 2 : 0) | (p.out2x ? 4 : 0);
       switch (flavour) {
         case 0: epi_role_conv<false, false, false>(p, x); break;
@@ -726,21 +673,15 @@ __global__ void __launch_bounds__(DUAL ? 192 : NUM_THREADS) __maxnreg__(DUAL ? 1
     } else
     for (int t = blockIdx.x; t < total_tiles; t += gridDim.x, ++it) {
       const int acc = it & (p.n_acc - 1);
-      if (p.epi_tile_split && !one_group && (it & 1) != half) continue;  // the other warp group owns this tile
+      if (p.epi_tile_split && (it & 1) != half) continue;  // the other warp group owns this tile
       const TileCoord c = decode_tile(p, t);
       const uint32_t acc_ph = (uint32_t)(it >> p.acc_shift) & 1u;
 
-      const bool ts_on = leader && (e & 3) == 0 && (p.epi_tile_split || one_group || e == 0);
+      const bool ts_on = leader && (e & 3) == 0 && (p.epi_tile_split || e == 0);
       if (ts_on) Y5_TS(2, it, 0);
-      if (p.wait_suspend) ptx::mbar_wait_suspend(&tmem_full[acc], acc_ph);
-      else ptx::mbar_wait(&tmem_full[acc], acc_ph);
+      ptx::mbar_wait_suspend(&tmem_full[acc], acc_ph);
       ptx::tc_fence_after();
       if (ts_on) Y5_TS(2, it, 1);
-      if (p.dbg & 4) {
-        ptx::tc_fence_before();
-        ptx::mbar_arrive(&tmem_empty[acc]);
-        continue;
-      }
       for (int m = 0; m < p.m_sub; ++m) {  // the tile's 128-pixel sub-tiles, stacked along H
       const int hsub = c.h0 + m * p.Ht;
       const int h = hsub + hl, w = c.w0 + wl;
@@ -896,7 +837,7 @@ __global__ void __launch_bounds__(DUAL ? 192 : NUM_THREADS) __maxnreg__(DUAL ? 1
   __syncthreads();
   if (warp == 1) {
     ptx::tc_fence_after();
-    ptx::tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
+    ptx::tmem_dealloc(tmem_base, (uint32_t)TMEM_COLS);
   }
 }
 
@@ -927,7 +868,6 @@ CUtensorMapSwizzle swizzle_for(int bk) {
 struct ConvObj {
   ConvK k;
   int grid;
-  int threads;
   size_t smem;
   double flops;      // algorithmic 2*MACs
   double hbm_bytes;  // algorithmic in + out (+ residual) bytes
@@ -981,6 +921,9 @@ int y5obb_conv_create(const y5obb_conv_desc* d, y5obb_conv_t** out) {
   if (d->in_pix_stride % 8 || (reinterpret_cast<uintptr_t>(d->in) & 15)) return Y5OBB_EINVAL;
   if (d->KH < 1 || d->KW < 1 || d->pad_h < 0 || d->pad_w < 0) return Y5OBB_EINVAL;
   if (d->mode == MODE_CONV && d->act && !(d->flags & Y5OBB_CONV_BIAS_HALVED)) return Y5OBB_EINVAL;
+  constexpr int known_flags = Y5OBB_CONV_NO_ROWSHIFT | Y5OBB_CONV_NO_RESIDENT | Y5OBB_CONV_NO_PAIRW | Y5OBB_CONV_BIAS_HALVED |
+                              Y5OBB_CONV_NO_UP_TMA | Y5OBB_CONV_NO_RES_RED;
+  if (d->flags & ~known_flags) return Y5OBB_EINVAL;
   const int64_t in_row_stride = d->in_row_stride ? d->in_row_stride : d->in_pix_stride * d->Win;
   const int64_t in_img_stride = d->in_img_stride ? d->in_img_stride : in_row_stride * d->Hin;
   if (in_row_stride % 8 || in_img_stride % 8) return Y5OBB_EINVAL;
@@ -1026,22 +969,9 @@ int y5obb_conv_create(const y5obb_conv_desc* d, y5obb_conv_t** out) {
   const int det_rec_w = ((d->det_no - 180 + 1) + 3) / 4 * 4;  // compact record: (5 + nc + 1) floats rounded up to 4
   if (d->mode == MODE_DETECT && d->det_decode == 2)
     k.epi_stage_bytes = std::max<uint32_t>(EPI_STAGE_DET, (uint32_t)align_up((size_t)32 * det_rec_w * 4, 128));
-  // operand ring (+ resident weights): everything but the epilogue staging; `dual` = two CTAs per SM, each with half of it
-  // staging depth: in-kernel stamps show ~100 cycles between "accumulator loaded" and "staging buffer free" with two buffers per
-  // warp, i.e. the TMA stores are not what the epilogue waits for
-  k.wait_suspend = 1;
-  k.mma_loop = 0;
-  k.no_full_fence = 0;
-  k.res_prefetch = 0;  // measured neutral to slightly negative (op 4: 65.4 -> 67.6 us): opt-in
-  if (const char* rp = getenv("Y5OBB_RES_PREFETCH")) k.res_prefetch = atoi(rp) ? 1 : 0;
-  if (const char* nf = getenv("Y5OBB_NO_FULL_FENCE")) k.no_full_fence = atoi(nf) ? 1 : 0;
-  if (const char* ml = getenv("Y5OBB_MMA_LOOP")) k.mma_loop = atoi(ml) ? 1 : 0;
-  if (const char* ws = getenv("Y5OBB_WAIT_SUSPEND")) k.wait_suspend = atoi(ws) ? 1 : 0;
-  k.epi_bufs = 2;  // four buffers measured slower (they cost operand-ring depth): opt-in through Y5OBB_EPI_BUFS=4
-  if (const char* eb = getenv("Y5OBB_EPI_BUFS")) k.epi_bufs = (atoi(eb) == 4 && d->mode == MODE_CONV) ? 4 : 2;
   const size_t bias_bytes = align_up((size_t)(cout_pad + 32) * 4, 128);  // the bias lives in shared memory behind the staging buffers
-  size_t SMEM_BUDGET = (size_t)SMEM_TOTAL - 1024 - (size_t)EPI_WARPS * k.epi_bufs * k.epi_stage_bytes - bias_bytes;
-  const size_t BUDGET_ONE = SMEM_BUDGET, BUDGET_DUAL = (size_t)DUAL_SMEM - 1024 - (size_t)4 * k.epi_bufs * k.epi_stage_bytes - bias_bytes;
+  // operand ring (+ resident weights): everything but the epilogue staging and the bias
+  const size_t SMEM_BUDGET = (size_t)SMEM_TOTAL - 1024 - (size_t)EPI_WARPS * EPI_BUFS * k.epi_stage_bytes - bias_bytes;
   // Row-shift mode (stride-1 convs with KH > 1): an 8 x 16 pixel tile whose A stage holds Ht + KH - 1 image
   // rows; the KH vertical taps read the same stage at row offsets that are whole 8-row swizzle groups, so each
   // input row crosses L2 -> shared memory (Ht + KH - 1) / Ht times per kw instead of KH times.  Taken when the
@@ -1092,10 +1022,9 @@ int y5obb_conv_create(const y5obb_conv_desc* d, y5obb_conv_t** out) {
     // small units share a stage: every mbarrier round trip (~300-500 cycles in the two single-thread loops)
     // then moves >= ~24 KB
     int group = 1;
-    if (!(d->flags & Y5OBB_CONV_NO_GROUP))
-      while (group < k.n_units && group < 4 && (size_t)(group + 1) * unit_bytes <= 40 * 1024 &&
-             (SMEM_BUDGET - k.b_res_bytes) / ((size_t)(group + 1) * unit_bytes) >= 3)
-        ++group;
+    while (group < k.n_units && group < 4 && (size_t)(group + 1) * unit_bytes <= 40 * 1024 &&
+           (SMEM_BUDGET - k.b_res_bytes) / ((size_t)(group + 1) * unit_bytes) >= 3)
+      ++group;
     k.group = group;
     stage_bytes = unit_bytes * group;
     k.stages = (int)std::min<size_t>(MAX_STAGES, (SMEM_BUDGET - k.b_res_bytes) / stage_bytes);
@@ -1104,59 +1033,15 @@ int y5obb_conv_create(const y5obb_conv_desc* d, y5obb_conv_t** out) {
   const bool want_rowshift = d->stride == 1 && d->KH > 1 && Wout >= 8 && !(d->flags & Y5OBB_CONV_NO_ROWSHIFT);
   const int sub_cols = bn <= 32 ? 32 : (bn <= 64 ? 64 : (bn <= 128 ? 128 : 256));
   {
-    // Configuration search.  dual (two CTAs per SM: 256 TMEM columns and half the shared memory each, 4 epilogue warps) is
-    // preferred whenever a 3-deep ring fits: its two pipelines hide each other's hand-shake latencies.  Within a configuration
-    // the largest m_sub whose accumulator stages fit the TMEM columns (two stages; one is enough in dual mode, where the other
-    // CTA overlaps the epilogue), that keeps every SM busy and adds no edge waste along H.  Y5OBB_CONV_MSUB1 / Y5OBB_CONV_NO_DUAL
-    // and the environment variables Y5OBB_MSUB_MAX / Y5OBB_DUAL (0 / 1) pin the choice for A-B runs.
-    int m_max = 4;
-    if (d->flags & Y5OBB_CONV_MSUB1) m_max = 1;
-    if (const char* e = getenv("Y5OBB_MSUB_MAX")) m_max = std::max(1, std::min(4, atoi(e)));
-    // MEASURED NEGATIVE (profiles/r2_occupancy.txt, r2_dual_experiment.txt): the runtime grants ONE resident CTA per SM to these
-    // kernels whatever their register / shared-memory footprint (even wgrad_kernel: 47 registers, 60 KB), so the dual
-    // configuration only runs as two waves of half-sized CTAs and loses 5-30 % on most layers.  It stays off unless
-    // Y5OBB_DUAL is set (1: if the occupancy query grants two CTAs; 2: unconditionally), and is kept for the A-B record.
-    int dual_ok = 0;
-    int dual_force = 0;
-    if (const char* e = getenv("Y5OBB_DUAL")) {
-      dual_ok = atoi(e) ? 1 : 0;
-      dual_force = atoi(e) == 2;  // 2: skip the runtime's occupancy answer (experiment)
-    }
-    if (dual_ok && dual_force) {
-      cudaFuncSetAttribute(conv_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DUAL_SMEM);
-      cudaFuncSetAttribute(conv_tc_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    }
-    if (dual_ok && !dual_force) {  // the two CTAs must really fit together (registers: 192 threads x the kernel's count)
-      static int dual_fits = -1;
-      if (dual_fits < 0) {
-        int nb = 0;
-        cudaFuncSetAttribute(conv_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DUAL_SMEM);
-        cudaFuncSetAttribute(conv_tc_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, conv_tc_kernel<true>, 64 + 4 * 32, DUAL_SMEM) != cudaSuccess) {
-          (void)cudaGetLastError();
-          nb = 0;
-        }
-        dual_fits = nb >= 2 ? 1 : 0;
-      }
-      dual_ok = dual_fits;
-    }
+    // Configuration search: the largest m_sub whose two accumulator stages fit the TMEM columns, that keeps every SM busy and
+    // adds no edge waste along H (m_sub = 1 only has to fit); row-shift before one load per tap.
     bool ok = false;
-    for (int dual = dual_ok; dual >= 0 && !ok; --dual) {
-      SMEM_BUDGET = dual ? BUDGET_DUAL : BUDGET_ONE;
-      const int cols = dual ? 256 : 512;
-      for (int m = 4; m >= 1 && !ok; m >>= 1) {
-        if (m > m_max || m * sub_cols * (dual ? 1 : 2) > cols) continue;
-        for (int rs = want_rowshift ? 1 : 0; rs >= 0 && !ok; --rs) {
-          if (!plan(rs == 1, m)) continue;
-          const long long tiles = (long long)k.n_tiles_m * nt;
-          const bool busy = tiles >= (long long)sm_count() * (dual ? 2 : 1);
-          const bool enough = (m == 1 && !dual) || (busy && Hout % (k.Ht * m) == 0 && k.stages >= 3);
-          ok = enough;
-          if (ok) {
-            k.epi_warps = dual ? 4 : 8;
-            k.tmem_cols = cols;
-          }
-        }
+    for (int m = 4; m >= 1 && !ok; m >>= 1) {
+      if (m * sub_cols * 2 > TMEM_COLS) continue;
+      for (int rs = want_rowshift ? 1 : 0; rs >= 0 && !ok; --rs) {
+        if (!plan(rs == 1, m)) continue;
+        const long long tiles = (long long)k.n_tiles_m * nt;
+        ok = m == 1 || (tiles >= sm_count() && Hout % (k.Ht * m) == 0 && k.stages >= 3);
       }
     }
     if (!ok) {
@@ -1168,14 +1053,9 @@ int y5obb_conv_create(const y5obb_conv_desc* d, y5obb_conv_t** out) {
   k.sub_cols = sub_cols;
   k.acc_stride = sub_cols * k.m_sub;
   k.a_sub16 = (uint32_t)(BM * bk * 2) >> 4;
-  k.n_acc = std::min(MAX_ACC, k.tmem_cols / k.acc_stride);
-  if (d->flags & Y5OBB_CONV_ACC2) k.n_acc = 2;
+  k.n_acc = std::min(MAX_ACC, TMEM_COLS / k.acc_stride);
   k.acc_shift = 0;
   while ((1 << k.acc_shift) < k.n_acc) ++k.acc_shift;
-  {
-    const char* e = getenv("Y5OBB_NO_PDL");
-    k.pdl = ((d->flags & Y5OBB_CONV_NO_PDL) || (e && e[0] == '1')) ? 0 : 1;
-  }
   k.fd_ntn = make_fastdiv((uint32_t)k.n_tiles_n);
   k.fd_per_img = make_fastdiv((uint32_t)(k.tiles_h * k.tiles_w));
   k.fd_tiles_w = make_fastdiv((uint32_t)k.tiles_w);
@@ -1193,13 +1073,11 @@ int y5obb_conv_create(const y5obb_conv_desc* d, y5obb_conv_t** out) {
   // In-place residual (the Bottleneck chain: out = chain = res): the add can be done by the TMA store itself (a bf16 reduce-add at
   // L2), which removes the epilogue's residual loads - they queue behind the producer's outstanding TMA loads (2-3 k cycles) and
   // bounded the residual layers.  The sum is then rounded twice (conv + SiLU to bf16, then the bf16 add) instead of once.
-  // (Y5OBB_RES_RED=0 or the flag Y5OBB_CONV_NO_RES_RED: the epilogue loads the residual and adds in fp32, one rounding)
+  // (the flag Y5OBB_CONV_NO_RES_RED: the epilogue loads the residual and adds in fp32, one rounding)
   k.res_red = (d->res && d->res == d->out && d->res_pix_stride == d->out_pix_stride && !d->out2x && !(d->flags & Y5OBB_CONV_NO_RES_RED) &&
                (!geom || (d->res_row_stride == d->out_row_stride && d->res_img_stride == d->out_img_stride)))
                   ? 1
                   : 0;
-  if (const char* rr = getenv("Y5OBB_RES_RED"))
-    if (!atoi(rr)) k.res_red = 0;
   k.out2x = static_cast<__nv_bfloat16*>(d->out2x);
   k.out2x_pix_stride = d->out2x_pix_stride;
   k.det_out = d->det_out;
@@ -1225,7 +1103,6 @@ int y5obb_conv_create(const y5obb_conv_desc* d, y5obb_conv_t** out) {
   k.pairw = (d->stride == 2 && !(d->Win & 1) && in_row_stride == d->in_pix_stride * d->Win &&
              !(d->flags & Y5OBB_CONV_NO_PAIRW)) ? 1 : 0;
   k.in_pix_stride = (int)d->in_pix_stride;
-  k.dbg = (d->flags >> 8) & 7;
   {  // activations: (C, W, H, B), element strides (1, s, s, 1)
     cuuint64_t dims[4] = {(cuuint64_t)d->Cin, (cuuint64_t)d->Win, (cuuint64_t)d->Hin, (cuuint64_t)d->B};
     cuuint64_t strides[3] = {(cuuint64_t)d->in_pix_stride * 2, (cuuint64_t)in_row_stride * 2,
@@ -1337,25 +1214,20 @@ int y5obb_conv_create(const y5obb_conv_desc* d, y5obb_conv_t** out) {
     }
   }
   const int total = k.n_tiles_m * k.n_tiles_n;
-  o->grid = std::min(total, sm_count() * (k.epi_warps == 4 ? 2 : 1));
+  o->grid = std::min(total, sm_count());
   if (k.b_resident && k.n_tiles_n > 1) o->grid = o->grid / k.n_tiles_n * k.n_tiles_n;  // one N tile per CTA (resident weights)
-  o->threads = 64 + 32 * k.epi_warps;
   // many tiles per CTA: the two epilogue groups alternate tiles (two epilogues in flight, any BN);
   // few tiles per CTA: they split the columns of each tile (shortest single-tile latency)
-  k.epi_tile_split = (total >= 4 * o->grid && k.epi_warps == 8) ? 1 : 0;
-  if (d->mode == MODE_DETECT && d->det_decode == 2 && k.epi_warps == 8) k.epi_tile_split = 1;  // a record is assembled by one thread over all columns
+  k.epi_tile_split = total >= 4 * o->grid ? 1 : 0;
+  if (d->mode == MODE_DETECT && d->det_decode == 2) k.epi_tile_split = 1;  // a record is assembled by one thread over all columns
   // >= 116 KB so that two CTAs (each owning all 512 TMEM columns) can never share an SM
-  o->smem = k.b_res_bytes + (size_t)k.stages * stage_bytes + (size_t)k.epi_warps * k.epi_bufs * k.epi_stage_bytes + bias_bytes + 1024;
-  if (k.epi_warps == 8) o->smem = std::max<size_t>(o->smem, 116 * 1024);
-  else if (o->smem > (size_t)DUAL_SMEM) {
-    delete o;
-    return Y5OBB_EINVAL;
-  }
+  o->smem = k.b_res_bytes + (size_t)k.stages * stage_bytes + (size_t)EPI_WARPS * EPI_BUFS * k.epi_stage_bytes + bias_bytes + 1024;
+  o->smem = std::max<size_t>(o->smem, 116 * 1024);
   o->flops = 2.0 * d->B * Hout * Wout * (double)d->Cout * d->Cin * d->KH * d->KW;
   o->hbm_bytes = 2.0 * d->B * ((double)d->Hin * d->Win * (d->hbm_cin ? d->hbm_cin : d->Cin) + (double)Hout * Wout * d->Cout * (d->res ? 2 : 1));
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(conv_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_TOTAL);
+    cudaError_t e = cudaFuncSetAttribute(conv_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_TOTAL);
     if (e != cudaSuccess) {
       delete o;
       return cuda_fail(e);
@@ -1369,26 +1241,20 @@ int y5obb_conv_create(const y5obb_conv_desc* d, y5obb_conv_t** out) {
 int y5obb_conv_run(const y5obb_conv_t* conv, void* stream) {
   if (!conv) return Y5OBB_EINVAL;
   const ConvObj* o = reinterpret_cast<const ConvObj*>(conv);
-  if (o->k.pdl) {
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3((unsigned)o->grid);
-    cfg.blockDim = dim3((unsigned)o->threads);
-    cfg.dynamicSmemBytes = o->smem;
-    cfg.stream = (cudaStream_t)stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    cudaError_t e = o->k.epi_warps == 4 ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<true>, o->k)
-                                        : cudaLaunchKernelEx(&cfg, conv_tc_kernel<false>, o->k);
-    if (e != cudaSuccess) return cuda_fail(e);
-    return Y5OBB_OK;
-  }
-  if (o->k.epi_warps == 4) conv_tc_kernel<true><<<o->grid, o->threads, o->smem, (cudaStream_t)stream>>>(o->k);
-  else conv_tc_kernel<false><<<o->grid, o->threads, o->smem, (cudaStream_t)stream>>>(o->k);
-  Y5_LAUNCH_CHECK();
+  // programmatic dependent launch: the kernel's prologue overlaps the previous kernel's tail (griddepcontrol.wait in the kernel)
+  cudaLaunchConfig_t cfg;
+  memset(&cfg, 0, sizeof(cfg));
+  cfg.gridDim = dim3((unsigned)o->grid);
+  cfg.blockDim = dim3((unsigned)NUM_THREADS);
+  cfg.dynamicSmemBytes = o->smem;
+  cfg.stream = (cudaStream_t)stream;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = at;
+  cfg.numAttrs = 1;
+  cudaError_t e = cudaLaunchKernelEx(&cfg, conv_tc_kernel, o->k);
+  if (e != cudaSuccess) return cuda_fail(e);
   return Y5OBB_OK;
 }
 
@@ -1406,26 +1272,6 @@ int y5obb_conv_info(const y5obb_conv_t* conv, double* flops, double* hbm_bytes, 
 }
 
 void y5obb_conv_destroy(y5obb_conv_t* conv) { delete reinterpret_cast<ConvObj*>(conv); }
-
-int y5obb_conv_debug_occupancy(int dual, int threads, size_t dyn_smem, int* blocks_per_sm, int* regs, int* static_smem) {
-  if (!blocks_per_sm || !regs || !static_smem) return Y5OBB_EINVAL;
-  cudaFuncAttributes fa;
-  cudaError_t e;
-  if (dual) {
-    cudaFuncSetAttribute(conv_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DUAL_SMEM);
-    cudaFuncSetAttribute(conv_tc_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    e = cudaFuncGetAttributes(&fa, conv_tc_kernel<true>);
-    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, conv_tc_kernel<true>, threads, dyn_smem);
-  } else {
-    cudaFuncSetAttribute(conv_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_TOTAL);
-    e = cudaFuncGetAttributes(&fa, conv_tc_kernel<false>);
-    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, conv_tc_kernel<false>, threads, dyn_smem);
-  }
-  if (e != cudaSuccess) return cuda_fail(e);
-  *regs = fa.numRegs;
-  *static_smem = (int)fa.sharedSizeBytes;
-  return Y5OBB_OK;
-}
 
 int y5obb_conv_debug_timestamps(y5obb_conv_t* conv, unsigned long long* dev_buf_768) {
   if (!conv) return Y5OBB_EINVAL;

@@ -639,9 +639,8 @@ int nms_impl(const float* dets, const float* scores, const int32_t* image_ids, i
     Y5_CUDA(cudaFuncSetAttribute(k_reduce, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
     smem_set = 200 * 1024;
   }
-  // >= 640 blocks of 64 boxes in an image: a cluster of RC CTAs shares the scan (env Y5OBB_NMS_NO_CLUSTER=1 keeps the single CTA)
-  static const bool no_cluster = [] { const char* e = getenv("Y5OBB_NMS_NO_CLUSTER"); return e && e[0] == '1'; }();
-  if (!no_cluster && (max_per_image + TB - 1) / TB >= 640) {  // measured break-even ~40 k boxes (one barrier per 64-row block)
+  // >= 640 blocks of 64 boxes in an image: a cluster of RC CTAs shares the scan
+  if ((max_per_image + TB - 1) / TB >= 640) {  // measured break-even ~40 k boxes (one barrier per 64-row block)
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
     cfg.gridDim = dim3((unsigned)n_images * RC);
@@ -1164,7 +1163,7 @@ using namespace y5obb;
 
 extern "C" {
 
-int y5obb_abi_version(void) { return 1; }
+int y5obb_abi_version(void) { return 2; }
 int y5obb_last_cuda_error(void) { return g_last_cuda_error; }
 const char* y5obb_build_info(void) { return "liby5obb sm_100a " __DATE__ " " __TIME__; }
 

@@ -14,7 +14,6 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)_
 __device__ __forceinline__ void st_shared_f32(uint32_t addr, float v) {
   asm volatile("st.shared.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory");
 }
-__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 __device__ __forceinline__ float4 ld_shared_v4(uint32_t addr) {
   float4 v;
   asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));

@@ -12,7 +12,6 @@
 #include <cuda_bf16.h>
 
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 
@@ -25,7 +24,6 @@ namespace {
 constexpr int WG_THREADS = 192;
 constexpr int WG_MAX_STAGES = 8;
 constexpr int WG_SMEM = 200 * 1024;
-constexpr int WG_DUAL_SMEM = 110 * 1024;  // per CTA when two share an SM
 // a pixel block (= one TMA box per 64-channel chunk) has bk = 64, 128 or 256 pixels; a chunk is [bk pixels][128 B]
 
 struct WgradK {
@@ -47,7 +45,6 @@ struct WgradK {
   float* dW;                // element (tap, co, ci) at dW[tap * s_tap + row(co) * s_co + ci * s_ci]
   long long s_tap, s_co, s_ci;
   int co_group, co_group_pad;
-  int dbg;                  // timing experiments only (Y5OBB_WGRAD_DBG env; results are garbage): 1 = no TMA, 2 = no MMA
 };
 
 // MN-major, 128B-swizzled operand: 64-channel chunks of [pixels][128 B]; 8-pixel groups 1024 B apart (SBO), chunks
@@ -123,27 +120,23 @@ __global__ void __launch_bounds__(WG_THREADS, 1) wgrad_kernel(const __grid_const
       for (int st = s0; st < s1; ++st) {
         ptx::mbar_wait(&empty_bar[s], ph ^ 1u);
         uint8_t* sbase = smem + (size_t)s * p.stage_bytes;
-        if (p.dbg & 1) {
-          ptx::mbar_arrive(&full_bar[s]);
-        } else {
-          ptx::mbar_expect_tx(&full_bar[s], tx);
-          for (int pb = 0; pb < p.PB; ++pb) {
-            const int k = st * p.PB + pb;        // pixel block; blocks past the end decode to b >= B: all zero fill
-            const int b = k / per_img;
-            const int r = k - b * per_img;
-            const int th = r / p.tiles_w;
-            const int ho0 = th * p.khp, wo0 = (r - th * p.tiles_w) * p.kwp;
-            uint8_t* sa = sbase + (size_t)pb * blk_bytes;
-            for (int c = 0; c < a_chunks; ++c)
-              ptx::tma_load_4d(sa + (size_t)c * WG_CHUNK, &p.tmA, &full_bar[s], cob * 128 + c * 64, wo0, ho0, b);
-            for (int t = 0; t < ntap; ++t) {
-              const int tap = tap0 + t;
-              const int kh = tap / p.KW, kw = tap - kh * p.KW;
-              const int wi0 = wo0 * p.stride + kw - p.pad_w, hi0 = ho0 * p.stride + kh - p.pad_h;
-              uint8_t* sb = sa + a_bytes + (size_t)t * b_bytes;
-              for (int c = 0; c < p.b_chunks; ++c)
-                ptx::tma_load_4d(sb + (size_t)c * WG_CHUNK, &p.tmB, &full_bar[s], cib * p.BN + c * 64, wi0, hi0, b);
-            }
+        ptx::mbar_expect_tx(&full_bar[s], tx);
+        for (int pb = 0; pb < p.PB; ++pb) {
+          const int k = st * p.PB + pb;        // pixel block; blocks past the end decode to b >= B: all zero fill
+          const int b = k / per_img;
+          const int r = k - b * per_img;
+          const int th = r / p.tiles_w;
+          const int ho0 = th * p.khp, wo0 = (r - th * p.tiles_w) * p.kwp;
+          uint8_t* sa = sbase + (size_t)pb * blk_bytes;
+          for (int c = 0; c < a_chunks; ++c)
+            ptx::tma_load_4d(sa + (size_t)c * WG_CHUNK, &p.tmA, &full_bar[s], cob * 128 + c * 64, wo0, ho0, b);
+          for (int t = 0; t < ntap; ++t) {
+            const int tap = tap0 + t;
+            const int kh = tap / p.KW, kw = tap - kh * p.KW;
+            const int wi0 = wo0 * p.stride + kw - p.pad_w, hi0 = ho0 * p.stride + kh - p.pad_h;
+            uint8_t* sb = sa + a_bytes + (size_t)t * b_bytes;
+            for (int c = 0; c < p.b_chunks; ++c)
+              ptx::tma_load_4d(sb + (size_t)c * WG_CHUNK, &p.tmB, &full_bar[s], cib * p.BN + c * 64, wi0, hi0, b);
           }
         }
         if (++s == p.stages) {
@@ -164,25 +157,23 @@ __global__ void __launch_bounds__(WG_THREADS, 1) wgrad_kernel(const __grid_const
       for (int st = s0; st < s1; ++st) {
         ptx::mbar_wait(&full_bar[s], ph);
         ptx::tc_fence_after();
-        if (!(p.dbg & 2)) {
-          for (int pb = 0; pb < p.PB; ++pb) {
-            const uint32_t sa = ring + (uint32_t)s * p.stage_bytes + (uint32_t)pb * blk_bytes;
-            const uint64_t da = desc_hi | (uint64_t)((sa & 0x3FFFFu) >> 4);
-            // up to 4 chunks (N = 256) per instruction: the dz tile (A) is fetched once for all of them
-            for (int c0 = 0, g = 0; c0 < nchunks; c0 += 4, ++g) {
-              const int nn = min(4, nchunks - c0);
-              const uint32_t sb = sa + a_bytes + (uint32_t)c0 * WG_CHUNK;
-              const uint64_t db = desc_hi | (uint64_t)((sb & 0x3FFFFu) >> 4);
-              const uint32_t d_tmem = tmem_base + (uint32_t)(c0 * 64);
-              const uint32_t idesc = p.idesc | ((uint32_t)(nn * 8) << 17);
-              uint32_t accumulate = (started >> g) & 1u;
+        for (int pb = 0; pb < p.PB; ++pb) {
+          const uint32_t sa = ring + (uint32_t)s * p.stage_bytes + (uint32_t)pb * blk_bytes;
+          const uint64_t da = desc_hi | (uint64_t)((sa & 0x3FFFFu) >> 4);
+          // up to 4 chunks (N = 256) per instruction: the dz tile (A) is fetched once for all of them
+          for (int c0 = 0, g = 0; c0 < nchunks; c0 += 4, ++g) {
+            const int nn = min(4, nchunks - c0);
+            const uint32_t sb = sa + a_bytes + (uint32_t)c0 * WG_CHUNK;
+            const uint64_t db = desc_hi | (uint64_t)((sb & 0x3FFFFu) >> 4);
+            const uint32_t d_tmem = tmem_base + (uint32_t)(c0 * 64);
+            const uint32_t idesc = p.idesc | ((uint32_t)(nn * 8) << 17);
+            uint32_t accumulate = (started >> g) & 1u;
 #pragma unroll 4
-              for (int j = 0; j < nk; ++j) {  // 16 pixel rows = 2048 B per MMA
-                ptx::umma_bf16(d_tmem, da + (uint64_t)(128 * j), db + (uint64_t)(128 * j), idesc, accumulate);
-                accumulate = 1u;
-              }
-              started |= 1u << g;
+            for (int j = 0; j < nk; ++j) {  // 16 pixel rows = 2048 B per MMA
+              ptx::umma_bf16(d_tmem, da + (uint64_t)(128 * j), db + (uint64_t)(128 * j), idesc, accumulate);
+              accumulate = 1u;
             }
+            started |= 1u << g;
           }
         }
         ptx::umma_commit(&empty_bar[s]);
@@ -209,7 +200,7 @@ __global__ void __launch_bounds__(WG_THREADS, 1) wgrad_kernel(const __grid_const
       ptx::tc_fence_after();
       const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16);
       const int ncols = min(p.BN, p.Cin - cib * p.BN);
-      if (cob * 128 + q * 32 < p.Cout && !(p.dbg & 2)) {  // warp-uniform
+      if (cob * 128 + q * 32 < p.Cout) {  // warp-uniform
         for (int t = 0; t < ntap; ++t) {
           float* row = p.dW + (long long)(tap0 + t) * p.s_tap + (long long)co_row * p.s_co + (long long)(cib * p.BN) * p.s_ci;
           for (int c0 = 0; c0 < ncols; c0 += 16) {  // chunk (c0 / 64) of tap t starts at TMEM column (t * b_chunks) * 64
@@ -305,7 +296,6 @@ int y5obb_wgrad_create(const y5obb_wgrad_desc* d, y5obb_wgrad_t** out) {
   }
   k.co_group = d->co_group;
   k.co_group_pad = d->co_group_pad;
-  if (const char* e = getenv("Y5OBB_WGRAD_DBG")) k.dbg = atoi(e);
   k.ci_blks = (d->Cin + 255) / 256;
   k.BN = ((d->Cin + k.ci_blks - 1) / k.ci_blks + 15) / 16 * 16;
   k.b_chunks = (k.BN + 63) / 64;
@@ -322,19 +312,6 @@ int y5obb_wgrad_create(const y5obb_wgrad_desc* d, y5obb_wgrad_t** out) {
   int best_T = std::min(ntaps, 8 / k.b_chunks);
   while (best_T > 1 && (uint32_t)(k.a_chunks + best_T * k.b_chunks) * (uint32_t)best_bk * 128 > WG_SMEM / 2) --best_T;
   if ((uint32_t)(k.a_chunks + best_T * k.b_chunks) * (uint32_t)best_bk * 128 > WG_SMEM / 2) best_bk = 64;
-  if (const char* e = getenv("Y5OBB_WGRAD_BK")) {  // experiments
-    const int v = atoi(e);
-    if (v == 64 || v == 128 || v == 256) {
-      best_bk = v;
-      best_T = std::min(ntaps, 8 / k.b_chunks);
-      while (best_T > 1 && (uint32_t)(k.a_chunks + best_T * k.b_chunks) * (uint32_t)v * 128 > WG_SMEM / 2) --best_T;
-    }
-  }
-  if (const char* e = getenv("Y5OBB_WGRAD_T")) best_T = std::max(1, std::min(atoi(e), std::min(ntaps, 8 / k.b_chunks)));
-  if (best_bk == 0) {
-    delete o;
-    return Y5OBB_EINVAL;
-  }
   k.bk = best_bk;
   k.chunk = (uint32_t)best_bk * 128;
   // pixel block kwp x khp = bk output pixels: the shape that covers the map with the fewest blocks (ties: widest rows)
@@ -366,19 +343,10 @@ int y5obb_wgrad_create(const y5obb_wgrad_desc* d, y5obb_wgrad_t** out) {
   k.steps = k.nblocks;
   k.tmem_cols = 64;
   while (k.tmem_cols < (uint32_t)(k.T * k.b_chunks * 64)) k.tmem_cols <<= 1;
-  // Two CTAs per SM (each <= 256 TMEM columns and <= 112 KB of shared memory) whenever a 3-deep ring still fits: the two
-  // producer / MMA / epilogue pipelines hide each other's hand-shake latencies (no unit of a single pipeline is above ~45 %
-  // busy, profiles/r2_conv_ncu_summary.txt).  Experimental: Y5OBB_WGRAD_DUAL=1 switches it on.
-  bool dual = k.tmem_cols <= 256 && 3 * (size_t)k.stage_bytes + 2048 <= WG_DUAL_SMEM;
-  {  // measured: no gain (the runtime keeps these kernels at one resident CTA per SM, profiles/r2_occupancy.txt): opt-in only
-    const char* e = getenv("Y5OBB_WGRAD_DUAL");
-    dual = dual && e && atoi(e) != 0;
-  }
-  if (dual) k.stages = (int)std::min<size_t>(WG_MAX_STAGES, (WG_DUAL_SMEM - 2048) / k.stage_bytes);
   const int items = k.ngroups * k.co_blks * k.ci_blks;
   {  // split-K: minimise (waves) x (steps per CTA + the fixed cost of a CTA: TMEM alloc, pipeline fill, fp32 atomic
      // epilogue - about 512 pixels' worth of pipeline steps); 1 CTA per SM
-    const int sms = sm_count() * (dual ? 2 : 1);  // CTAs in flight
+    const int sms = sm_count();  // CTAs in flight
     const int fixed = std::max(1, 512 / k.bk);
     long long best_cost2 = -1;
     int bestk = 1;
@@ -426,8 +394,7 @@ int y5obb_wgrad_create(const y5obb_wgrad_desc* d, y5obb_wgrad_t** out) {
     }
   }
   o->grid = items * k.ksplit;
-  o->smem = (size_t)k.stages * k.stage_bytes + 1024;
-  if (!dual) o->smem = std::max<size_t>(o->smem, 116 * 1024);  // one CTA per SM: it may own all 512 TMEM columns
+  o->smem = std::max<size_t>((size_t)k.stages * k.stage_bytes + 1024, 116 * 1024);  // one CTA per SM: it may own all 512 TMEM columns
   o->flops = 2.0 * d->B * d->Ho * d->Wo * (double)d->Cout * d->Cin * d->KH * d->KW;
   static bool attr_set = false;
   if (!attr_set) {
@@ -448,18 +415,6 @@ int y5obb_wgrad_run(const y5obb_wgrad_t* w, void* stream) {
   const WgradObj* o = reinterpret_cast<const WgradObj*>(w);
   wgrad_kernel<<<o->grid, WG_THREADS, o->smem, (cudaStream_t)stream>>>(o->k);
   Y5_LAUNCH_CHECK();
-  return Y5OBB_OK;
-}
-
-int y5obb_wgrad_debug_occupancy(size_t dyn_smem, int* blocks_per_sm, int* regs) {
-  if (!blocks_per_sm || !regs) return Y5OBB_EINVAL;
-  cudaFuncAttributes fa;
-  cudaFuncSetAttribute(wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, WG_SMEM + 2048);
-  cudaFuncSetAttribute(wgrad_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-  cudaError_t e = cudaFuncGetAttributes(&fa, wgrad_kernel);
-  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, wgrad_kernel, WG_THREADS, dyn_smem);
-  if (e != cudaSuccess) return cuda_fail(e);
-  *regs = fa.numRegs;
   return Y5OBB_OK;
 }
 

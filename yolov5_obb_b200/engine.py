@@ -150,12 +150,8 @@ class InferenceEngine:
                 out[i] = Slice.full(new(hw[i][0], hw[i][1], ch[i]))
 
         self.out_slices = out   # per top-level layer: where its output lives (tests read them for teacher-forced parity)
-        import os
-        dbg_no_res = os.environ.get("Y5OBB_DEBUG_NO_RES") == "1"  # timing experiments only (wrong results)
 
         def add_conv(x, w, b, k, s, p, act, dst: Optional[Slice] = None, res=None, out2x=None, detd=None):
-            if dbg_no_res:
-                res = None
             wp, bp = pack_weights(w.cpu(), b.cpu(), MODE_DETECT if detd else 0, detd["no"] if detd else 0)   # packed on the host
             if act and not detd:
                 bp = bp * 0.5   # the SiLU epilogue wants 0.5 * bias (Y5OBB_CONV_BIAS_HALVED)

@@ -11,7 +11,6 @@ statically when the plan is built (first writer of a channel range overwrites).
 Parameter gradients land in views of ONE flat fp32 buffer owned by the plan (run() returns it); the autograd
 Function in yolo.py hands them to autograd, which accumulates into `.grad` (so GradScaler / DDP hooks see them).
 """
-import os
 from typing import Dict, List, Optional
 
 import torch
@@ -70,8 +69,8 @@ class BackwardPlan:
         # re-mapping copies at the end - so wgrad_kernel (tensor-bound, one 60 KB CTA per SM) shares the SMs with the
         # HBM-bound BatchNorm backward passes and fills the tails of the dgrad launches.  Every wgrad reads buffers nothing
         # writes after its producer (its own dz, the saved activation) and accumulates into its own slice of the flat
-        # gradient buffer, so only the interleaving changes.  Y5OBB_WGRAD_STREAM=0 keeps everything on one stream.
-        self.side = torch.cuda.Stream(dev) if os.environ.get("Y5OBB_WGRAD_STREAM", "1") == "1" else None
+        # gradient buffer, so only the interleaving changes.
+        self.side = torch.cuda.Stream(dev)
         self.prof = None  # set to {} to collect per-step-kind device times (ms) during run()
 
         def add(tag, fn):
@@ -253,7 +252,7 @@ class BackwardPlan:
                     op, wp = add_dgrad(Slice.full(dz), w_d, k, k - 1 - p, gx, "dgrad")
                     part["dgrad_wp"] = wp
                     self.keep.append(op)
-                elif k == 3 and p == 1 and x.H % 2 == 0 and x.W % 2 == 0 and os.environ.get("Y5OBB_DGRAD_S2", "phase") == "phase":
+                elif k == 3 and p == 1 and x.H % 2 == 0 and x.W % 2 == 0:
                     # Output pixels of parity (ph, pw) only see the taps of matching parity: four 1- / 2-tap stride-1
                     # convolutions of dz, each written to every other pixel of gx - 9 tap-GEMMs per 4 outputs instead of
                     # the 36 of the zero-stuffed form.
@@ -331,7 +330,7 @@ class BackwardPlan:
         det = eng.model.model[-1]
         with torch.no_grad():
             self.flat.zero_()
-            if self.prof is None and self.side is not None:
+            if self.prof is None:
                 cur, side = torch.cuda.current_stream(eng.device), self.side
                 side.wait_stream(cur)                       # fork (after the flat buffer was zeroed)
                 for tag, step in self.steps:
@@ -344,9 +343,6 @@ class BackwardPlan:
                     else:
                         step(st)
                 cur.wait_stream(side)                       # join: the copies below read the weight gradients
-            elif self.prof is None:
-                for _, step in self.steps:
-                    step(st)
             else:  # debug: CUDA events around every step, summed per kind (and listed per wgrad / dgrad layer)
                 evs = []
                 for tag, step in self.steps:
