@@ -175,6 +175,13 @@ int y5obb_stem_s2d(const float* x_nchw, void* out_nhwc16, int B, int H, int W, i
 /* same for a uint8 image, with the caller-side `/ 255` (train.py:299, val.py:187-188) folded in */
 int y5obb_stem_s2d_u8(const uint8_t* x_nchw, void* out_nhwc16, int B, int H, int W, int pad_cols, void* stream);
 int y5obb_sppf_pool(void* buf, int64_t pix_stride, int B, int H, int W, int C, void* stream);
+/* y5obb_stem_s2d_u8 for B tiles cropped from a whole scene, replacing the host crop-and-pad of
+ * DOTA_devkit/ImgSplit_multi_process.py:122-132 (saveimagepatches, rate 1) and the channel flip of cv2.imread's BGR pixels.
+ * scene_hwc [H][W][3] uint8 BGR (any H, W); origins2 [B][2] int32 (left, up) of each tile x tile window; tile b >= n_valid is
+ * written as zeros, as are pixels outside the scene.  out_nhwc16 as y5obb_stem_s2d with H = W = tile.  Bit-identical to
+ * flipping and zero-padding the crops on the host and calling y5obb_stem_s2d_u8. */
+int y5obb_stem_s2d_scene_u8(const uint8_t* scene_hwc, int H, int W, const int32_t* origins2, int B, int n_valid, int tile,
+                            void* out_nhwc16, int pad_cols, void* stream);
 
 /* ---- loss ------------------------------------------------------------------------------------
  * Replaces utils/loss.py:122-192 (ComputeLoss.__call__), :194-275 (build_targets) and utils/metrics.py:201-236
@@ -351,6 +358,28 @@ size_t y5obb_poly_nms_workspace_bytes(int64_t n);
 int y5obb_poly_nms_f64(const double* dets9, int64_t n, double thresh, int64_t* keep_out, int64_t* n_keep_out, void* workspace,
                        size_t workspace_bytes, void* stream);
 int y5obb_poly_iou_pairs_f64(const double* p8, const double* q8, double* iou_out, int64_t n, void* stream);
+
+/* ---- whole-scene merge of tile detections (double precision) ------------------------------------------------------
+ * y5obb_tiles_to_scene_f64 replaces DOTA_devkit/ResultMerge_multi_process.py:175-182 (poly2origpoly, rate 1) over the
+ * rbox2poly of val.py:226-232 / utils/rboxs_utils.py:106-126: det7 [n_tiles][max_det][7] (cx, cy, l, s, theta, conf, cls;
+ * the packed output of y5obb_nms_obb_f32) with counts[t] valid rows, tile origins2 [n_tiles][2] int32 (left, up) and
+ * scene_of [n_tiles] int32 (< 0: padding tile, its rows are ignored) -> dets9_out [n][9] (scene-space polygon + score, tile
+ * after tile, row after row; capacity n_tiles * max_det) and seg_out [n] = scene * nc + class.  *n_out = n and
+ * seg_hist_out [n_scenes * nc] = rows per segment, on the device.
+ * y5obb_poly_nms_segmented_f64 replaces ResultMerge_multi_process.py:183-236 (mergesingle: py_cpu_nms_poly_fast, :62-123,
+ * once per (scene, class) file entry): y5obb_poly_nms_f64 run independently on every segment seg_id[i] in
+ * [0, n_segments).  seg_counts_host [n_segments] (HOST) = rows per segment, which must match seg_id; it sizes the
+ * workspace.  keep_out [n]: kept indices into dets9, segment after segment, each in descending score (ties: lower index
+ * first); segment s owns keep_out[seg_offsets_out[s] .. seg_offsets_out[s + 1]).  Y5OBB_EINVAL when a segment has more
+ * than 1 638 400 rows (its mask row would not fit the 200 KB shared-memory scan). */
+size_t y5obb_tiles_to_scene_workspace_bytes(int n_tiles);
+int y5obb_tiles_to_scene_f64(const float* det7, const int64_t* counts, int n_tiles, int max_det, const int32_t* origins2,
+                             const int32_t* scene_of, int n_scenes, int nc, double* dets9_out, int32_t* seg_out,
+                             int64_t* n_out, int64_t* seg_hist_out, void* workspace, size_t workspace_bytes, void* stream);
+size_t y5obb_poly_nms_segmented_workspace_bytes(const int64_t* seg_counts_host, int64_t n_segments);
+int y5obb_poly_nms_segmented_f64(const double* dets9, const int32_t* seg_id, int64_t n, const int64_t* seg_counts_host,
+                                 int64_t n_segments, double thresh, int64_t* keep_out, int64_t* seg_offsets_out,
+                                 void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- post-NMS geometry + validation matching (SURVEY 8f rank 3) ------------------------------------------------------
  * One launch per batch for val.py:226-250 + process_batch (val.py:69-92): detections pred7 [batch, max_det, 7] (the packed

@@ -69,6 +69,12 @@ PROTOTYPES = {
     "y5obb_poly_nms_workspace_bytes": (c_size_t, [c_int64]),
     "y5obb_poly_nms_f64": (c_int, [c_void_p, c_int64, ctypes.c_double, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "y5obb_poly_iou_pairs_f64": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
+    "y5obb_tiles_to_scene_workspace_bytes": (c_size_t, [c_int]),
+    "y5obb_tiles_to_scene_f64": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p,
+                                         c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "y5obb_poly_nms_segmented_workspace_bytes": (c_size_t, [c_void_p, c_int64]),
+    "y5obb_poly_nms_segmented_f64": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, ctypes.c_double, c_void_p,
+                                             c_void_p, c_void_p, c_size_t, c_void_p]),
     "y5obb_poly_nms_f32_workspace_bytes": (c_size_t, [c_int64]),
     "y5obb_poly_nms_f32": (c_int, [c_void_p, c_int64, c_float, c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "y5obb_poly_overlaps_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
@@ -88,6 +94,7 @@ PROTOTYPES = {
     "y5obb_detect_grad_pack": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "y5obb_stem_s2d": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "y5obb_stem_s2d_u8": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
+    "y5obb_stem_s2d_scene_u8": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p]),
     "y5obb_sppf_pool": (c_int, [c_void_p, c_int64, c_int, c_int, c_int, c_int, c_void_p]),
 }
 

@@ -6,8 +6,10 @@
 //   y5obb_sppf_pool    the three chained 5x5/s1/p2 max-pools of SPPF (models/common.py:181-196) in one
 //                      pass: y1 = 5x5, y2 = 9x9, y3 = 13x13 windows of x (max-pool composition), written
 //                      at channel offsets C, 2C, 3C of the same buffer (the torch.cat disappears).
-// Algorithmic bytes: stem_s2d reads 12*H*W fp32 and writes H*W/4 * 32 B per image; sppf_pool reads
-// H*W*C*2 and writes 3x that.
+//   y5obb_stem_s2d_scene_u8  the same layout pass for tiles cropped from a whole HWC BGR uint8 scene (channel flip, zero
+//                      padding outside the scene and for invalid tiles), so a DOTA scene never goes through host crops.
+// Algorithmic bytes: stem_s2d reads 12*H*W fp32 and writes H*W/4 * 32 B per image; stem_s2d_scene_u8 reads 3 B and writes
+// 8 B per tile pixel; sppf_pool reads H*W*C*2 and writes 3x that.  All three are HBM-bound.
 #include <cuda_bf16.h>
 
 #include <algorithm>
@@ -16,6 +18,21 @@
 
 namespace y5obb {
 namespace {
+
+// The pack-and-store tail of every stem layout pass: the 12 space-to-depth values of output pixel (row r = b * Ho + ho,
+// column wo) plus 4 zero channels -> 16 bf16 (round to nearest), one 32-byte store.  Destination rows carry pad_cols zero
+// pixels on each side (written once at allocation, never here).
+__device__ __forceinline__ void s2d_store(float (&v)[16], __nv_bfloat16* __restrict__ out, long long r, int Wo, int wo,
+                                          int pad_cols) {
+  v[12] = v[13] = v[14] = v[15] = 0.f;
+  uint4 o[2];
+  __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(o);
+#pragma unroll
+  for (int e = 0; e < 8; ++e) h[e] = __floats2bfloat162_rn(v[2 * e], v[2 * e + 1]);
+  uint4* dst = reinterpret_cast<uint4*>(out + ((r * (Wo + 2 * pad_cols)) + wo + pad_cols) * 16);
+  dst[0] = o[0];
+  dst[1] = o[1];
+}
 
 __global__ void k_stem_s2d(const float* __restrict__ x, __nv_bfloat16* __restrict__ out, int B, int H, int W,
                            int pad_cols) {
@@ -37,15 +54,7 @@ __global__ void k_stem_s2d(const float* __restrict__ x, __nv_bfloat16* __restric
       v[2 * 3 + c] = bot.x;  // (dy=1, dx=0)
       v[3 * 3 + c] = bot.y;  // (dy=1, dx=1)
     }
-    v[12] = v[13] = v[14] = v[15] = 0.f;
-    uint4 o[2];
-    __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(o);
-#pragma unroll
-    for (int e = 0; e < 8; ++e) h[e] = __floats2bfloat162_rn(v[2 * e], v[2 * e + 1]);
-    // destination rows carry pad_cols zero pixels on each side (written once at allocation, never here)
-    uint4* dst = reinterpret_cast<uint4*>(out + ((r * (Wo + 2 * pad_cols)) + wo + pad_cols) * 16);
-    dst[0] = o[0];
-    dst[1] = o[1];
+    s2d_store(v, out, r, Wo, wo, pad_cols);
   }
 }
 
@@ -71,15 +80,39 @@ __global__ void k_stem_s2d_u8(const uint8_t* __restrict__ x, __nv_bfloat16* __re
       v[2 * 3 + c] = (float)bot.x / 255.0f;
       v[3 * 3 + c] = (float)bot.y / 255.0f;
     }
-    v[12] = v[13] = v[14] = v[15] = 0.f;
-    uint4 o[2];
-    __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(o);
+    s2d_store(v, out, r, Wo, wo, pad_cols);
+  }
+}
+
+// Whole-scene form (DOTA_devkit/ImgSplit_multi_process.py:122-132 saveimagepatches at rate 1, then the caller-side `/ 255`):
+// tile b of the batch is the tile x tile window at origins[b] = (left, up) of an HWC BGR uint8 scene, as cv2.imread returns
+// it; model channel c is scene channel 2 - c; pixels outside the scene (the devkit's zero padding at the bottom and right)
+// and every tile b >= n_valid are zero.  Bit-identical to cropping on the host and running k_stem_s2d_u8.
+__global__ void k_stem_s2d_scene_u8(const uint8_t* __restrict__ scene, int H, int W, const int* __restrict__ origins, int B,
+                                    int n_valid, int tile, __nv_bfloat16* __restrict__ out, int pad_cols) {
+  const int Ho = tile >> 1, Wo = tile >> 1;
+  const long long total = (long long)B * Ho * Wo;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int wo = (int)(i % Wo);
+    const long long r = i / Wo;
+    const int ho = (int)(r % Ho);
+    const int b = (int)(r / Ho);
+    float v[16];
+    const bool valid = b < n_valid;
+    const int left = valid ? origins[2 * b] : 0, up = valid ? origins[2 * b + 1] : 0;
 #pragma unroll
-    for (int e = 0; e < 8; ++e) h[e] = __floats2bfloat162_rn(v[2 * e], v[2 * e + 1]);
-    // destination rows carry pad_cols zero pixels on each side (written once at allocation, never here)
-    uint4* dst = reinterpret_cast<uint4*>(out + ((r * (Wo + 2 * pad_cols)) + wo + pad_cols) * 16);
-    dst[0] = o[0];
-    dst[1] = o[1];
+    for (int dy = 0; dy < 2; ++dy) {
+      const int y = up + 2 * ho + dy;
+#pragma unroll
+      for (int dx = 0; dx < 2; ++dx) {
+        const int x = left + 2 * wo + dx;
+        const bool in = valid && y >= 0 && y < H && x >= 0 && x < W;
+        const uint8_t* p = scene + ((long long)y * W + x) * 3;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) v[(dy * 2 + dx) * 3 + c] = (float)(in ? p[2 - c] : (uint8_t)0) / 255.0f;
+      }
+    }
+    s2d_store(v, out, r, Wo, wo, pad_cols);
   }
 }
 
@@ -193,6 +226,20 @@ int y5obb_stem_s2d_u8(const uint8_t* x_nchw, void* out_nhwc16, int B, int H, int
   const long long total = (long long)B * (H / 2) * (W / 2);
   const int grid = (int)std::min<long long>((total + 255) / 256, (long long)sm_count() * 16);
   k_stem_s2d_u8<<<grid, 256, 0, (cudaStream_t)stream>>>(x_nchw, static_cast<__nv_bfloat16*>(out_nhwc16), B, H, W, pad_cols);
+  Y5_LAUNCH_CHECK();
+  return Y5OBB_OK;
+}
+
+int y5obb_stem_s2d_scene_u8(const uint8_t* scene_hwc, int H, int W, const int32_t* origins2, int B, int n_valid, int tile,
+                            void* out_nhwc16, int pad_cols, void* stream) {
+  if (!scene_hwc || !out_nhwc16 || H <= 0 || W <= 0 || B <= 0 || n_valid < 0 || n_valid > B || tile <= 0 || (tile & 1) ||
+      pad_cols < 0 || (n_valid > 0 && !origins2))
+    return Y5OBB_EINVAL;
+  if ((reinterpret_cast<uintptr_t>(origins2) & 7) || (reinterpret_cast<uintptr_t>(out_nhwc16) & 15)) return Y5OBB_EINVAL;
+  const long long total = (long long)B * (tile / 2) * (tile / 2);
+  const int grid = (int)std::min<long long>((total + 255) / 256, (long long)sm_count() * 16);
+  k_stem_s2d_scene_u8<<<grid, 256, 0, (cudaStream_t)stream>>>(scene_hwc, H, W, origins2, B, n_valid, tile,
+                                                              static_cast<__nv_bfloat16*>(out_nhwc16), pad_cols);
   Y5_LAUNCH_CHECK();
   return Y5OBB_OK;
 }

@@ -8,6 +8,7 @@
 #include <algorithm>
 
 #include "common.cuh"
+#include "rbox_poly.cuh"
 
 namespace y5obb {
 namespace {
@@ -15,20 +16,7 @@ namespace {
 __global__ void k_rbox2poly(const float* __restrict__ r, float* __restrict__ p, int64_t n) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const float cx = r[5 * i], cy = r[5 * i + 1], w = r[5 * i + 2], h = r[5 * i + 3], th = r[5 * i + 4];
-  const float c = cosf(th), s = sinf(th);
-  const float w2 = __fdiv_rn(w, 2.0f), h2 = __fdiv_rn(h, 2.0f);
-  const float v1x = __fmul_rn(w2, c), v1y = __fmul_rn(-w2, s);   // vector1 = (w/2 * Cos, -w/2 * Sin)
-  const float v2x = __fmul_rn(-h2, s), v2y = __fmul_rn(-h2, c);  // vector2 = (-h/2 * Sin, -h/2 * Cos)
-  float* o = p + 8 * i;
-  o[0] = __fadd_rn(__fadd_rn(cx, v1x), v2x);  // point1 = center + vector1 + vector2
-  o[1] = __fadd_rn(__fadd_rn(cy, v1y), v2y);
-  o[2] = __fsub_rn(__fadd_rn(cx, v1x), v2x);  // point2 = center + vector1 - vector2
-  o[3] = __fsub_rn(__fadd_rn(cy, v1y), v2y);
-  o[4] = __fsub_rn(__fsub_rn(cx, v1x), v2x);  // point3 = center - vector1 - vector2
-  o[5] = __fsub_rn(__fsub_rn(cy, v1y), v2y);
-  o[6] = __fadd_rn(__fsub_rn(cx, v1x), v2x);  // point4 = center - vector1 + vector2
-  o[7] = __fadd_rn(__fsub_rn(cy, v1y), v2y);
+  rbox_to_poly(r[5 * i], r[5 * i + 1], r[5 * i + 2], r[5 * i + 3], r[5 * i + 4], p + 8 * i);
 }
 
 __global__ void k_poly2hbb(const float* __restrict__ p, float* __restrict__ hbb, int64_t n) {

@@ -12,6 +12,7 @@
 // one detection) go to the lower label index; the reference's numpy quicksort leaves them unspecified.
 // HBM-bound: 28 B read + (niou + 48) B written per detection; the label list of an image lives in shared memory.
 #include "common.cuh"
+#include "rbox_poly.cuh"  // rbox_to_poly: utils/rboxs_utils.py:106-126 (torch branch)
 
 namespace y5obb {
 namespace {
@@ -33,22 +34,6 @@ struct VmArgs {
   float* hbbn;             // [B, max_det, 4] native-space xyxy boxes (pred_hbbn) or null
   int* overflow;           // set to 1 if an image has more than VM_MAX_LABELS labels
 };
-
-// utils/rboxs_utils.py:106-126 (torch branch), as csrc/rbox_utils.cu k_rbox2poly
-__device__ __forceinline__ void rbox_to_poly(float cx, float cy, float w, float h, float th, float* o) {
-  const float c = cosf(th), s = sinf(th);
-  const float w2 = __fdiv_rn(w, 2.0f), h2 = __fdiv_rn(h, 2.0f);
-  const float v1x = __fmul_rn(w2, c), v1y = __fmul_rn(-w2, s);
-  const float v2x = __fmul_rn(-h2, s), v2y = __fmul_rn(-h2, c);
-  o[0] = __fadd_rn(__fadd_rn(cx, v1x), v2x);
-  o[1] = __fadd_rn(__fadd_rn(cy, v1y), v2y);
-  o[2] = __fsub_rn(__fadd_rn(cx, v1x), v2x);
-  o[3] = __fsub_rn(__fadd_rn(cy, v1y), v2y);
-  o[4] = __fsub_rn(__fsub_rn(cx, v1x), v2x);
-  o[5] = __fsub_rn(__fsub_rn(cy, v1y), v2y);
-  o[6] = __fadd_rn(__fsub_rn(cx, v1x), v2x);
-  o[7] = __fadd_rn(__fsub_rn(cy, v1y), v2y);
-}
 
 // poly2hbb (utils/rboxs_utils.py:147-165) then xywh2xyxy (utils/general.py:555-562): note x1 = xc - w/2, not x_min
 __device__ __forceinline__ void poly_to_xyxy(const float* p, float* b) {

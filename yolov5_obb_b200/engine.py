@@ -271,20 +271,58 @@ class InferenceEngine:
                 x = x.contiguous().float()
                 _lib.check(L.y5obb_stem_s2d(x.data_ptr(), self.x_s2d.data_ptr(), self.B, self.H, self.W, 1, st),
                            "y5obb_stem_s2d")
-            # the layer sequence is fixed (same buffers every call): from the third call on it is replayed as one CUDA
-            # graph - the layout pass above stays outside because it reads the caller's tensor (Y5OBB_NO_GRAPH=1 disables)
-            self._calls += 1
-            if self._use_graph and self._calls > 2:
-                if self._graph is None:
-                    torch.cuda.synchronize(self.device)
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g, capture_error_mode="thread_local"):
-                        self._run_ops(_lib.stream_ptr(self.device))
-                    self._graph = g
-                self._graph.replay()
-            else:
-                self._run_ops(st)
+            self._replay()
         return self.pred
+
+    def forward_tiles(self, scene, origins: torch.Tensor, n_valid) -> torch.Tensor:
+        """Runs the plan on B tiles cropped from whole scenes on the device (DOTA_devkit/ImgSplit_multi_process.py:226-273 at
+        rate 1, without the patch files): scene is one uint8 [H, W, 3] BGR tensor (cv2.imread's layout) or a list of them,
+        origins an int32 [B, 2] device tensor of tile (left, up), n_valid the number of tiles cut from each scene (an int, or
+        one per scene; their tiles are consecutive in origins).  Tiles after the last valid one are zero.  Pixels outside a
+        scene are zero (the devkit's padding), channels are flipped to RGB and scaled by 1/255 exactly as forward() does for a
+        uint8 batch.  Returns the same engine-owned buffer as forward()."""
+        scenes = [scene] if isinstance(scene, torch.Tensor) else list(scene)
+        counts = [int(n_valid)] if isinstance(n_valid, int) else [int(k) for k in n_valid]
+        if self.H != self.W or len(scenes) != len(counts) or not scenes:
+            raise RuntimeError("forward_tiles needs a square plan and one tile count per scene")
+        if tuple(origins.shape) != (self.B, 2) or origins.dtype != torch.int32 or not origins.is_contiguous():
+            raise RuntimeError(f"origins must be a contiguous int32 [{self.B}, 2] tensor")
+        _lib.require_cuda(origins, "origins")
+        if any(k < 0 for k in counts) or sum(counts) > self.B:
+            raise RuntimeError(f"tile counts {counts} do not fit a batch of {self.B}")
+        st = _lib.stream_ptr(self.device)
+        L = _lib.lib()
+        with torch.cuda.device(self.device):
+            b0 = 0
+            for s, k in zip(scenes, counts):
+                _lib.require_cuda(s, "scene")
+                if s.dtype != torch.uint8 or s.dim() != 3 or s.shape[2] != 3 or not s.is_contiguous():
+                    raise RuntimeError("a scene must be a contiguous uint8 [H, W, 3] tensor")
+                if k:
+                    _lib.check(L.y5obb_stem_s2d_scene_u8(s.data_ptr(), s.shape[0], s.shape[1], origins[b0].data_ptr(), k, k,
+                                                         self.H, self.x_s2d[b0].data_ptr(), 1, st), "y5obb_stem_s2d_scene_u8")
+                b0 += k
+            if b0 < self.B:   # padding tiles: zeros (no scene pixel is read)
+                _lib.check(L.y5obb_stem_s2d_scene_u8(scenes[0].data_ptr(), 1, 1, origins.data_ptr(), self.B - b0, 0, self.H,
+                                                     self.x_s2d[b0].data_ptr(), 1, st), "y5obb_stem_s2d_scene_u8")
+            self._replay()
+        return self.pred
+
+    def _replay(self):
+        """The op list after the layout pass: the layer sequence is fixed (same buffers every call), so from the third call on
+        it is replayed as one CUDA graph - the layout pass stays outside because it reads the caller's tensor
+        (Y5OBB_NO_GRAPH=1 disables)."""
+        self._calls += 1
+        if self._use_graph and self._calls > 2:
+            if self._graph is None:
+                torch.cuda.synchronize(self.device)
+                g = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(g, capture_error_mode="thread_local"):
+                    self._run_ops(_lib.stream_ptr(self.device))
+                self._graph = g
+            self._graph.replay()
+        else:
+            self._run_ops(_lib.stream_ptr(self.device))
 
     def _run_ops(self, st):
         for op in self.ops:

@@ -329,15 +329,30 @@ class Model(nn.Module):
         graph): batches in flight on DIFFERENT streams must use different slots (pipeline.DetectPipeline does)."""
         if self.training:
             raise RuntimeError("detect_records is an inference entry point (model.eval())")
-        from .engine import InferenceEngine
         from .general import DetectRecords
-        key = ("records", tuple(x.shape), x.device.index) + ((int(slot),) if slot else ())
+        eng = self._records_engine(tuple(x.shape), x.device, slot)
+        return DetectRecords(eng.forward(x), eng.nc)
+
+    def detect_records_tiles(self, scene, origins, n_valid, tile: int, slot: int = 0):
+        """detect_records on tiles cut from whole scenes on the device (InferenceEngine.forward_tiles): scene a uint8
+        [H, W, 3] BGR tensor or a list of them, origins int32 [B, 2] (left, up) on their device, n_valid tiles per scene (an
+        int or one per scene), the rest of the batch padding.  Runs the plan detect_records uses for a [B, 3, tile, tile]
+        batch (same buffers, same captured graph) and returns its records."""
+        if self.training:
+            raise RuntimeError("detect_records_tiles is an inference entry point (model.eval())")
+        from .general import DetectRecords
+        eng = self._records_engine((origins.shape[0], 3, int(tile), int(tile)), origins.device, slot)
+        return DetectRecords(eng.forward_tiles(scene, origins, n_valid), eng.nc)
+
+    def _records_engine(self, shape, device, slot):
+        from .engine import InferenceEngine
+        key = ("records", tuple(shape), device.index) + ((int(slot),) if slot else ())
         eng = self._engines.get(key)
         sig = self._weights_signature()
         if eng is None or eng._weights_sig != sig:
-            eng = self._engines[key] = InferenceEngine(self, x.shape[0], x.shape[2], x.shape[3], x.device, compact_detect=True)
+            eng = self._engines[key] = InferenceEngine(self, shape[0], shape[2], shape[3], device, compact_detect=True)
             eng._weights_sig = sig
-        return DetectRecords(eng.forward(x), eng.nc)
+        return eng
 
     def _weights_signature(self):
         tr = getattr(self, "_sig_tensors", None)
